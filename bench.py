@@ -3,6 +3,7 @@
 
     python bench.py --gpus 1 --steps 50 --warmup 10              # our sm_100a path, one JSON line
     python bench.py --impl reference --steps 5 --warmup 1        # the reference's CPU path (oracle port)
+    python bench.py --steps 50 --dump-outputs DIR                 # ... and write the last timed step's outputs as DIR/<name>.npy
     torchrun --nproc-per-node N ... bench.py --gpus N ...        # batch-sharded, one NCCL gradient all-reduce/step
 
 One "step" = y = conv(x); y.backward(g) producing dx, dweight, dbias for one batch of synthetic input
@@ -496,6 +497,28 @@ def run_reference(args):
     return 0
 
 
+DUMP_WHOLE_BYTES = 32 << 20    # an output larger than this is written as a fixed sample of DUMP_SAMPLE of its entries
+DUMP_SAMPLE = 1 << 21
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes what the timed step returned to its caller as out_dir/<name>.npy in float32 (complex: a trailing (real, imag) axis).
+    An output of more than DUMP_WHOLE_BYTES is written flat, as its entries at DUMP_SAMPLE positions drawn once with seed 0 and kept
+    in ascending order, so that two runs write the same positions.  At the headline shape y and dx are sampled (8 MB each), dweight
+    (18 MB) and dbias are whole."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        t = t.detach()
+        a = torch.view_as_real(t) if t.is_complex() else t
+        if a.numel() * 4 > DUMP_WHOLE_BYTES:
+            rows = a.reshape(-1, 2) if t.is_complex() else a.reshape(-1)
+            index = np.sort(np.random.default_rng(0).choice(rows.shape[0], size=DUMP_SAMPLE, replace=False))
+            a = rows[torch.from_numpy(index).to(rows.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), a.float().cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -533,12 +556,18 @@ def run_ours(args):
         reserved_sms = int(os.environ.get("SC_RESERVED_SMS", "12"))
         nb.get_plan(dev, (H, W), (H, W), conv.n_modes, conv.max_n_modes).set_reserved_sms(reserved_sms)
 
+    last = {}
+
     def step_body():
         conv.weight.tensor.grad = None
         conv.bias.grad = None
         x.grad = None
         y = conv(x)
         y.backward(g)
+        if args.dump_outputs:
+            # the output's storage (a graph replay rewrites it); detached, so that this step's autograd graph is still freed here and
+            # not while the next step is being captured
+            last["y"] = y.detach()
         if reducer is not None:
             reducer.finish()               # nothing pending (backward already ordered the stream after the collective): ends the step's bookkeeping
 
@@ -606,6 +635,8 @@ def run_ours(args):
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"y": last["y"], "dx": x.grad, "dweight": conv.weight.tensor.grad, "dbias": conv.bias.grad})
     launches = _lib.launch_count() - launches0
     if graph is not None:
         launches = launches_per_step * args.steps      # replayed by the graph: the library's own counter does not see them
@@ -833,7 +864,10 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the PyTorch+cuFFT denominator and the other BASELINE configs")
     ap.add_argument("--layer-only", action="store_true", help="internal: measure the Fourier layer (f1 / f2) and print LAYER_JSON")
     ap.add_argument("--no-graph", action="store_true", help="time the eager autograd path instead of a captured CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write y, dx, dweight, dbias of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.layer_only):
+        ap.error("--dump-outputs writes the outputs of the timed step of --impl ours")
     if args.layer_only:
         return run_layer(args)
     if args.impl == "reference":

@@ -1,8 +1,7 @@
 """Import the UNMODIFIED reference `neuralop/layers/spectral_convolution.py` in this container.
 
-TEST INFRASTRUCTURE ONLY -- used by `oracle/make_golden.py` to mint the golden vectors under
-`tests/golden/` and by `tests/test_oracle_vs_reference.py` (skipped where `/root/reference` does not
-exist, i.e. on the GPU box). Nothing in the product package imports this.
+TEST INFRASTRUCTURE ONLY -- used by the `oracle/make_golden*.py` generators to mint the stored vectors
+under `tests/golden/`. Neither the tests nor the product package import this.
 
 `neuralop/__init__.py` transitively needs h5py/zencfg/... (absent), so the parent packages are
 pre-seeded as empty namespace modules and only the one file (plus its three siblings

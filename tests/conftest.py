@@ -184,6 +184,36 @@ def load_fno_golden(name):
     return meta, io, params, grads
 
 
+_REFERENCE_CHECKS = {}
+
+
+def reference_checks(name="reference_checks"):
+    """(store, meta) of the stored reference results (oracle/make_golden_reference_checks.py): store = {key: (shape, largest
+    magnitude, values at the sampled positions)} of `name`.npz, meta = reference_checks.json with the module trees of
+    reference_swap_models.json.gz as meta["swap_models"]."""
+    if name not in _REFERENCE_CHECKS:
+        import gzip
+        from oracle.make_golden_reference_checks import load_store
+        with open(os.path.join(GOLDEN_DIR, "reference_checks.json")) as f:
+            meta = json.load(f)
+        with gzip.open(os.path.join(GOLDEN_DIR, "reference_swap_models.json.gz"), "rt") as f:
+            meta["swap_models"] = json.load(f)
+        _REFERENCE_CHECKS[name] = (load_store(os.path.join(GOLDEN_DIR, name + ".npz")), meta)
+    return _REFERENCE_CHECKS[name]
+
+
+def stored_rel_err(store, key, got):
+    """Largest difference between `got` and the reference tensor stored under `key`, at the stored positions, over the reference's
+    largest magnitude; also the difference of the two largest magnitudes, so that no entry of `got` can outgrow the reference's."""
+    from oracle.make_golden_reference_checks import sample_index
+    shape, absmax, values = store[key]
+    assert tuple(got.shape) == shape, (key, tuple(got.shape), shape)
+    got = got.detach().cpu()
+    flat = got.reshape(-1)[torch.from_numpy(sample_index(shape, key, values.shape[0]))].to(values.dtype)
+    peak = abs(float(got.abs().max()) - absmax) if got.numel() else 0.0
+    return max(float((flat - values).abs().max()) if values.numel() else 0.0, peak) / max(absmax, 1e-20)
+
+
 def build_fno_stack(meta, params, device=None):
     """lifting -> FNOBlocks -> projection from this package's drop-ins, as `FNO.__init__` builds them (fno.py:289-345, defaults:
     lifting / projection channel ratio 2), holding the golden's parameters.  Returns (modules dict, forward function)."""

@@ -1,14 +1,12 @@
 """The Fourier-layer oracle (oracle/fno_block_oracle.py) against golden vectors minted from the UNMODIFIED reference `FNOBlocks`
-(oracle/make_golden_block.py) and, where /root/reference exists (the build container), against the live class: forward, dx and the
-gradient of every parameter the layer touches.  CPU only."""
-import importlib
-
+(oracle/make_golden_block.py) and against stored results of the live class for fresh parameters: forward, dx and the gradient of
+every parameter the layer touches.  CPU only."""
 import pytest
 import torch
 
-from conftest import block_golden_index, block_oracle_kwargs, load_block_golden
+from conftest import block_golden_index, block_oracle_kwargs, load_block_golden, reference_checks, stored_rel_err
 from oracle import fno_block_oracle as BO
-from oracle.load_reference import load_reference_spectral_conv, reference_available
+from oracle.make_golden_reference_checks import seeded_tensors
 
 CASES = sorted(block_golden_index().keys())
 
@@ -33,31 +31,24 @@ def test_block_oracle_matches_golden(name):
         assert rel_err(g[pname], grads[pname]) < 2e-5, pname
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not present (GPU box)")
-@pytest.mark.parametrize("name", ["block_d2_default_mid", "block_d2_default_last", "block_d3_mid", "block_d2_tanh",
-                                  "block_d2_preactivation_mid", "block_d2_upsample", "block_d2_no_mlp_mid", "block_d2_tucker"])
+LIVE_CASES = ["block_d2_default_mid", "block_d2_default_last", "block_d3_mid", "block_d2_tanh", "block_d2_preactivation_mid",
+              "block_d2_upsample", "block_d2_no_mlp_mid", "block_d2_tucker"]
+
+
+@pytest.mark.parametrize("name", LIVE_CASES)
 def test_block_oracle_matches_live_reference(name):
-    """Fresh random parameters and inputs (not the stored ones) through the live reference class and the restatement."""
-    meta, io, _, _ = load_block_golden(name)
-    load_reference_spectral_conv()
-    fb = importlib.import_module("neuralop.layers.fno_block")
-    torch.manual_seed(99)
-    blk = fb.FNOBlocks(meta["in_channels"], meta["out_channels"], tuple(meta["n_modes"]), n_layers=meta["n_layers"], **meta["ctor"])
-    with torch.no_grad():
-        for pname, p in blk.named_parameters():
-            if "skips" in pname:
-                p.add_(0.2 * torch.randn_like(p))
-    x = torch.randn_like(io["x"]).requires_grad_(True)
-    kw = {k: tuple(v) for k, v in meta["forward"].items()}
-    y = blk(x, meta["index"], **kw)
-    gy = torch.randn_like(y)
-    y.backward(gy)
-    params = {k: v.detach() for k, v in blk.named_parameters()}
-    y2, dx2, g2 = BO.fno_block_fwd_bwd(x.detach(), params, meta["index"], gy, **block_oracle_kwargs(meta))
-    assert rel_err(y2, y.detach()) < 1e-6
-    assert rel_err(dx2, x.grad) < 1e-6
-    for pname, p in blk.named_parameters():
-        if p.grad is not None:
-            assert rel_err(g2[pname], p.grad) < 1e-6, pname
-        else:
-            assert pname not in g2
+    """Fresh random parameters and inputs (not the ones of the golden file), drawn from seeds, through the restatement, against what
+    the reference class returned for them (oracle/make_golden_reference_checks.py)."""
+    meta, io, params, _ = load_block_golden(name)
+    store, checks = reference_checks()
+    key = f"block_{name}"
+    params = seeded_tensors([(k, tuple(v.shape), v.dtype) for k, v in params.items()], 99)
+    gen = torch.Generator().manual_seed(100)
+    x = torch.randn(*io["x"].shape, generator=gen, dtype=io["x"].dtype)
+    gy = torch.randn(*store[f"{key}__y"][0], generator=gen, dtype=io["y"].dtype)
+    y2, dx2, g2 = BO.fno_block_fwd_bwd(x, params, meta["index"], gy, **block_oracle_kwargs(meta))
+    assert stored_rel_err(store, f"{key}__y", y2) < 1e-6
+    assert stored_rel_err(store, f"{key}__dx", dx2) < 1e-6
+    assert sorted(g2.keys()) == checks[key]["touched"]
+    for pname in checks[key]["touched"]:
+        assert stored_rel_err(store, f"{key}__g__{pname}", g2[pname]) < 1e-6, pname

@@ -1,20 +1,19 @@
 """fno_block_precision "half" / "mixed" (SURVEY section 8 f3) without a GPU.
 
 (1) The oracle's statement of the half-precision contraction (`contract_dense_half`: operands rounded to fp16, fp32 accumulation,
-    fp16 result) against the reference's own `einsum_complexhalf` (neuralop/layers/einsum_utils.py:10-36) run live on CPU -- the one
-    stage of the reduced-precision path that can execute here (the half FFTs need cuFFT).
+    fp16 result) against what the reference's own `einsum_complexhalf` (neuralop/layers/einsum_utils.py:10-36) returned on CPU -- the
+    one stage of the reduced-precision path that can execute there (the half FFTs need cuFFT).
 (2) The host logic of `_SpectralConvDenseReduced` -- where the tensors are rounded, what is saved, straight-through gradients --
     with the device primitives emulated (transforms: a trivial adjoint pair; contraction: einsum; rounding: the pointwise kernel's
     host check) against the same pipeline written with `oracle.round_half`."""
 import contextlib
-import importlib
 
 import pytest
 import torch
 
 from neuraloperator_b200 import _lib, spectral_conv as sc
 from oracle import spectral_conv_oracle as O
-from oracle.load_reference import load_reference_spectral_conv, reference_available
+from conftest import reference_checks, stored_rel_err
 
 
 def test_round_half_is_fp16_rounding_with_straight_through_gradient():
@@ -28,22 +27,26 @@ def test_round_half_is_fp16_rounding_with_straight_through_gradient():
     assert torch.equal(torch.view_as_real(rc), torch.view_as_real(c).half().float())
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not present (GPU box)")
-@pytest.mark.parametrize("shape", [(2, 3, 4, (5, 3)), (1, 8, 8, (6,)), (2, 4, 3, (3, 2, 4))])
-def test_half_contraction_restatement_against_live_einsum_complexhalf(shape):
+HALF_CASES = [(2, 3, 4, (5, 3)), (1, 8, 8, (6,)), (2, 4, 3, (3, 2, 4))]
+
+
+def half_case_inputs(shape):
     B, Ci, Co, kept = shape
-    load_reference_spectral_conv()
-    eu = importlib.import_module("neuralop.layers.einsum_utils")
     torch.manual_seed(3)
     xm = torch.randn(B, Ci, *kept, dtype=torch.complex64)
     w = torch.randn(Ci, Co, *kept, dtype=torch.complex64) / Ci ** 0.5
-    sym = "cdef"[: len(kept)]
-    eq = f"ab{sym},bz{sym}->az{sym}"                         # the string _contract_dense builds (spectral_convolution.py:21-40)
-    ref = eu.einsum_complexhalf(eq, xm.chalf(), w)           # the weight arrives as cfloat and is cast inside, as in the reference
-    ref = torch.view_as_complex(torch.view_as_real(ref).float())
+    return xm, w
+
+
+@pytest.mark.parametrize("shape", HALF_CASES)
+def test_half_contraction_restatement_against_live_einsum_complexhalf(shape):
+    """Against what the reference's einsum_complexhalf returned for these operands (stored by oracle/make_golden_reference_checks.py,
+    from the string _contract_dense builds, spectral_convolution.py:21-40, the weight passed as cfloat and cast inside)."""
+    store, _ = reference_checks()
+    xm, w = half_case_inputs(shape)
     ours = O.contract_dense_half(xm, w)
     # same operand rounding; the reference rounds each of the four real products to fp16 before combining them: <= 2 fp16 ulps apart
-    assert (ours - ref).abs().max() <= 2.0 ** -9 * ref.abs().max()
+    assert stored_rel_err(store, f"half{HALF_CASES.index(shape)}", ours) <= 2.0 ** -9
 
 
 class _Plan:

@@ -2,11 +2,13 @@
 :93-125) against `neuraloperator_b200.SpectralConv` WITHOUT a GPU: the whole parameter grid (4 factorizations x 2 implementations x
 separable x 1-4 dims x real / complex; Hermitian flag x dims x even / odd sizes x resolution scaling x modes) runs through the
 module's own host logic -- plan lookup, weight slicing, which chain runs, operand strides, mutable n_modes, output grids -- with the
-device primitives emulated by the oracle's torch.fft statements of the two transforms and by einsums for the contractions.  Where the
-live reference is importable, every result is ALSO compared with the unmodified reference class on the same weights.
+device primitives emulated by the oracle's torch.fft statements of the two transforms and by einsums for the contractions.  Every
+result is ALSO compared with what the unmodified reference class returned on the same weights (stored by
+oracle/make_golden_reference_checks.py).
 The GPU twin of this file is tests/test_gpu_zzz_a_reference_suite.py."""
 import contextlib
 import math
+import re
 
 import pytest
 import torch
@@ -14,7 +16,7 @@ import torch
 import neuraloperator_b200 as nb
 from neuraloperator_b200 import spectral_conv as sc
 from oracle import spectral_conv_oracle as O
-from oracle.load_reference import load_reference_spectral_conv, reference_available
+from conftest import reference_checks, stored_rel_err
 from test_factorized_host_logic import _LIB as _CHAIN_LIB, _pair_reduce, _table_contract
 
 
@@ -63,6 +65,10 @@ class _Lib(type(_CHAIN_LIB)):
 
 @pytest.fixture
 def emulated(monkeypatch):
+    return emulate_device(monkeypatch)
+
+
+def emulate_device(monkeypatch):
     lib = _Lib()
     monkeypatch.setattr(sc._lib, "load", lambda: lib)
     monkeypatch.setattr(sc._lib, "check", lambda rc, what: None)
@@ -89,19 +95,30 @@ def assert_close(a, b, tol):
     assert (a - b).abs().max().item() / max(b.abs().max().item(), 1e-20) < tol
 
 
-def _reference_twin(conv, **ctor):
-    """The unmodified reference class holding the same weight (reconstructed dense), or None when /root/reference is absent."""
-    if not reference_available():
-        return None
-    ref = load_reference_spectral_conv()
-    twin = ref.SpectralConv(conv.in_channels, conv.out_channels if not conv.separable else conv.in_channels,
-                            tuple(ctor.pop("user_modes")), bias=conv.bias is not None, factorization=None,
-                            implementation="reconstructed", separable=conv.separable, complex_data=conv.complex_data, **ctor)
-    with torch.no_grad():
-        twin.weight.tensor.copy_(conv.weight.to_tensor())
-        if conv.bias is not None:
-            twin.bias.copy_(conv.bias)
-    return twin
+def case_key(prefix, case, twin):
+    return f"{prefix}_{re.sub(r'[^0-9A-Za-z.]+', '_', str(case))}_{twin}"
+
+
+class StoredTwin:
+    """Stands for the unmodified reference class holding the same weight (reconstructed dense): `check` compares an output with what
+    that class returned for the same input, stored under the case's key, in the order the suite asks."""
+
+    def __init__(self, key):
+        self.key, self.n, self.n_modes = key, 0, None
+
+    def check(self, out, x, tol):
+        store, _ = reference_checks("reference_suite")
+        assert stored_rel_err(store, f"{self.key}__{self.n}", out) < tol
+        self.n += 1
+
+
+def _stored_twins(prefix, case):
+    made = []
+
+    def twin_of(conv, **ctor):
+        made.append(StoredTwin(case_key(prefix, case, len(made))))
+        return made[-1]
+    return twin_of
 
 
 FACTORIZATIONS = ["Dense", "CP", "Tucker", "TT"]
@@ -114,8 +131,8 @@ MODES, FEWER_MODES, SIDE = (10, 8, 6, 6), (6, 6, 4, 4), 12
 def suite_factorized_vs_dense(device, factorization, implementation, separable, dim, complex_data, tol, twin_of=None):
     """What the reference's `test_SpectralConv` (:7-90) asserts, for one point of its parameter grid, on `device`:
     a conv in any weight form equals its dense twin holding the reconstructed weight; shrinking `n_modes` at run time keeps the output
-    shape; a conv with resolution_scaling_factor 0.5 / 2 halves / doubles every spatial extent.  twin_of(conv, **ctor) may return the
-    unmodified reference module with the same weight: then every output is compared with it as well."""
+    shape; a conv with resolution_scaling_factor 0.5 / 2 halves / doubles every spatial extent.  twin_of(conv, **ctor) may return a
+    stand-in for the unmodified reference module with the same weight: then every output is checked against it as well."""
     torch.manual_seed(0)
     modes = MODES[:dim]
     make = lambda *a, **k: nb.SpectralConv(*a, **k).to(device)                                            # noqa: E731
@@ -132,13 +149,13 @@ def suite_factorized_vs_dense(device, factorization, implementation, separable, 
             assert_close(out, dense(x), tol)
         twin = twin_of(conv, user_modes=modes) if twin_of is not None else None
         if twin is not None:
-            assert_close(out, twin(x.cpu()).to(device), tol)
+            twin.check(out, x, tol)
         conv.n_modes = FEWER_MODES[:dim]                    # incremental training shrinks the modes at run time
         fewer = conv(x)
         assert fewer.shape == out.shape
         if twin is not None:
             twin.n_modes = FEWER_MODES[:dim]
-            assert_close(fewer, twin(x.cpu()).to(device), tol)
+            twin.check(fewer, x, tol)
         for factor, side in ((0.5, SIDE // 2), (2, SIDE * 2)):
             scaler = make(3, 4, modes, resolution_scaling_factor=factor)
             xr = torch.randn(2, 3, *(SIDE,) * dim, device=device)
@@ -146,12 +163,13 @@ def suite_factorized_vs_dense(device, factorization, implementation, separable, 
             assert res.shape[1] == 4 and list(res.shape[2:]) == [side] * dim
             twin = twin_of(scaler, user_modes=modes, resolution_scaling_factor=factor) if twin_of is not None else None
             if twin is not None:
-                assert_close(res, twin(xr.cpu()).to(device), tol)
+                twin.check(res, xr, tol)
 
 
-def suite_real_output_shapes(device, hermitian, dim, side, scaling, modes, tol, with_twin=False):
+def suite_real_output_shapes(device, hermitian, dim, side, scaling, modes, tol, twin_of=None):
     """The reference's `test_SpectralConv2` (:93-125): real float32 output of the right (rounded) size for even / odd grids, with and
-    without the Hermitian flag, at every resolution scaling."""
+    without the Hermitian flag, at every resolution scaling; checked against twin_of(conv) as above when given."""
+    torch.manual_seed(0)
     modes = modes[:dim]
     want = [side] * dim if scaling is None else [round(side * scaling)] * dim
     conv = nb.SpectralConv(3, 4, modes, enforce_hermitian_symmetry=hermitian, complex_data=False, resolution_scaling_factor=scaling).to(device)
@@ -159,21 +177,17 @@ def suite_real_output_shapes(device, hermitian, dim, side, scaling, modes, tol, 
     with torch.no_grad():
         res = conv(x)
     assert tuple(res.shape) == (2, 4, *want) and res.dtype == torch.float32 and not torch.is_complex(res)
-    if with_twin and reference_available():
-        ref = load_reference_spectral_conv()
-        twin = ref.SpectralConv(3, 4, modes, enforce_hermitian_symmetry=hermitian, complex_data=False, resolution_scaling_factor=scaling)
-        with torch.no_grad():
-            twin.weight.tensor.copy_(conv.weight.to_tensor())
-            twin.bias.copy_(conv.bias)
-            assert_close(res, twin(x.cpu()).to(device), tol)
+    if twin_of is not None:
+        twin_of(conv).check(res, x, tol)
 
 
 @pytest.mark.parametrize("factorization,implementation,separable,dim,complex_data", GRID_1)
 def test_SpectralConv(emulated, factorization, implementation, separable, dim, complex_data):
-    suite_factorized_vs_dense(torch.device("cpu"), factorization, implementation, separable, dim, complex_data, 2e-5, twin_of=_reference_twin)
+    suite_factorized_vs_dense(torch.device("cpu"), factorization, implementation, separable, dim, complex_data, 2e-5,
+                              twin_of=_stored_twins("g1", (factorization, implementation, separable, dim, complex_data)))
 
 
 @pytest.mark.parametrize("enforce_hermitian_symmetry,dim,spatial_size,resolution_scaling_factor,modes", GRID_2)
 def test_SpectralConv2(emulated, enforce_hermitian_symmetry, dim, spatial_size, modes, resolution_scaling_factor):
     suite_real_output_shapes(torch.device("cpu"), enforce_hermitian_symmetry, dim, spatial_size, resolution_scaling_factor, modes, 2e-5,
-                             with_twin=True)
+                             twin_of=_stored_twins("g2", (enforce_hermitian_symmetry, dim, spatial_size, resolution_scaling_factor, modes)))
