@@ -13,7 +13,9 @@
  * no CPU fallback behind any of them.
  *
  * Layouts (all contiguous, row-major):
- *   x, dx      float  (B, Ci, N_1..N_d)            input / its gradient
+ *   x, dx      float  (B, Ci, N_1..N_d)            input / its gradient; IEEE half or bfloat16 instead when the plan
+ *                                                  carries SC_FLAG_GRID_F16 / SC_FLAG_GRID_BF16 (the `float*` arguments
+ *                                                  then address 16-bit data)
  *   y, gy      float  (B, Co, M_1..M_d)            output / upstream gradient (M = N unless resampled)
  *   modes      sc_complex (B, C, k_1..k_d)         kept-mode block, ordered exactly like the reference's
  *                                                  x[slices_x] (:500-519): leading dims by increasing signed
@@ -48,12 +50,19 @@ typedef struct {
   int32_t n_modes[SC_MAX_DIMS];       /* SpectralConv.n_modes as STORED (last already n//2+1, :404-415)       */
   int32_t max_n_modes[SC_MAX_DIMS];   /* SpectralConv.max_n_modes = weight extents along the mode dims (:317-321) */
   int32_t fft_norm;                   /* SC_NORM_*                                                           */
-  int32_t flags;                      /* SC_FLAG_* (0 for SpectralConv.forward)                              */
+  int32_t flags;                      /* SC_FLAG_* (0 for SpectralConv.forward on float32 x)                 */
 } sc_problem;
 /* SC_FLAG_RESAMPLE: the synthesis places every kept SIGNED frequency f of a leading dim at bin (f mod M) of the output grid,
  * as neuralop/layers/resample.py:57-68 copies the spectrum corners (out_fft[..., -m//2:] = X[..., -m//2:]); without the flag
  * the unshifted spectrum is cropped / zero-padded at its end, as `ifftn(out_fft, s=...)` does in SpectralConv.forward (:548). */
 enum { SC_FLAG_RESAMPLE = 1 };
+/* SC_FLAG_GRID_F16 / SC_FLAG_GRID_BF16: the images on `grid` -- x, read by the forward analysis, and dx, written by the adjoint
+ * synthesis -- are stored as IEEE half / bfloat16 (what a model trained under torch.autocast feeds the conv).  Images on `out_grid`
+ * (y, gy) stay float.  The transforms compute in fp32 on the widened input, which every 16-bit value is exactly, so y equals the
+ * result for x converted to float bit for bit; dx is the fp32 adjoint rounded to nearest even.  The two flags exclude each other and
+ * SC_FLAG_RESAMPLE (sc_plan_create rejects those combinations before it touches a device); the tables do not depend on them, and
+ * the workspace sizes grow by one fp32 copy of the images on `grid`. */
+enum { SC_FLAG_GRID_F16 = 2, SC_FLAG_GRID_BF16 = 4 };
 
 /* ---- plan: kept-mode index set + twiddle tables (replaces the slices built at :465-519) ---------------- */
 int  sc_plan_create(const sc_problem* problem, sc_plan** plan_out);
@@ -275,6 +284,10 @@ int sc_hostcheck_channel_mix_act_backward(const float* gout, const float* pre, i
 int sc_hostcheck_channel_mix_weight_grad(const float* gpre, const float* in, float* dw, int32_t batch, int32_t in_channels,
                                          int32_t out_channels, int64_t n_points);
 int sc_hostcheck_pointwise(int op, const float* a, const float* b, float* out, int64_t n);
+/* The element conversion of the 16-bit image storage (`flag` = SC_FLAG_GRID_F16 or SC_FLAG_GRID_BF16), run on the host through the
+ * same __host__ __device__ pair the device kernels use.  to_16 == 0: n 16-bit values (uint16_t bit patterns) -> float; to_16 != 0:
+ * n floats -> 16-bit, round to nearest even (overflow to +-inf, NaN stays NaN). */
+int sc_hostcheck_convert(int flag, int to_16, const void* in, void* out, int64_t n);
 /* Dry run of sc_forward_cp / sc_backward_cp (kind 0, ranks[0] = R) or sc_forward_tt / sc_backward_tt (kind 1) for `problem` on a
  * host-only plan: every primitive launch of the chain is RECORDED instead of executed -- {opcode, n_args, args...} words, pointers as
  * integers over synthetic buffer addresses (region << 40; regions listed at the definition in csrc/sc_api.cu) -- so that the CPU test

@@ -12,6 +12,7 @@ from .build import LIB_PATH
 SC_MAX_DIMS = 4
 NORMS = {"forward": 0, "backward": 1, "ortho": 2}
 FLAG_RESAMPLE = 1
+FLAG_GRID_F16, FLAG_GRID_BF16 = 2, 4     # x / dx stored as float16 / bfloat16
 ACT_IDENTITY, ACT_GELU, ACT_RELU, ACT_SILU, ACT_TANH = 0, 1, 2, 3, 4
 POINTWISE_TANH, POINTWISE_TANH_BACKWARD, POINTWISE_ROUND_HALF, POINTWISE_ADD_I_TIMES, POINTWISE_MUL_NEG_I, POINTWISE_MUL = 0, 1, 2, 3, 4, 5
 
@@ -100,6 +101,7 @@ SIGNATURES = {
                                                       c_void_p, c_i32, c_i32, c_i64]),
     "sc_hostcheck_channel_mix_weight_grad": (c_int, [c_void_p, c_void_p, c_void_p, c_i32, c_i32, c_i32, c_i64]),
     "sc_hostcheck_pointwise": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_i64]),
+    "sc_hostcheck_convert": (c_int, [c_int, c_int, c_void_p, c_void_p, c_i64]),
     "sc_hostcheck_chain_log": (c_int, [c_void_p, c_int, c_int, c_i32, c_i32, c_i32, c_void_p, c_void_p, c_size_t, c_void_p]),
     "sc_probe_tma_gather": (c_int, [c_void_p, c_i32, c_i32, c_i64, c_void_p, c_void_p]),
     "sc_last_error": (ctypes.c_char_p, []),

@@ -91,6 +91,13 @@ static bool build_plan(const sc_problem& pr, Plan* p) {
   const int d = p->d;
   if (d < 1 || d > SC_MAX_DIMS) { set_error("ndim must be in 1..4"); return false; }
   if (pr.fft_norm < 0 || pr.fft_norm > 2) { set_error("unknown fft_norm"); return false; }
+  if ((pr.flags & SC_FLAG_GRID_F16) && (pr.flags & SC_FLAG_GRID_BF16)) {
+    set_error("SC_FLAG_GRID_F16 and SC_FLAG_GRID_BF16 exclude each other"); return false;
+  }
+  if ((pr.flags & (SC_FLAG_GRID_F16 | SC_FLAG_GRID_BF16)) && (pr.flags & SC_FLAG_RESAMPLE)) {
+    set_error("16-bit image storage (SC_FLAG_GRID_F16 / SC_FLAG_GRID_BF16) is not available with SC_FLAG_RESAMPLE"); return false;
+  }
+  p->grid16 = pr.flags & (SC_FLAG_GRID_F16 | SC_FLAG_GRID_BF16);
   if (!p->host_only && !cuda_ok(cudaGetDevice(&p->device), "cudaGetDevice")) return false;
 
   p->n_modes_total = p->grid_points = p->out_points = p->weight_elems_per_io = 1;
@@ -212,18 +219,24 @@ static int64_t chain_elems(const Plan* p, int64_t n_images) {
 struct Workspace {
   float2* buf[2];
   float2* modes[2];
+  float* grid32;     // 16-bit image storage only: the fp32 copy of x (analysis) or of dx (adjoint synthesis)
 };
+
+static size_t grid32_bytes(const Plan* p, int64_t n_images) {
+  return p->grid16 ? align256((size_t)(n_images * p->grid_points) * sizeof(float)) : 0;
+}
 
 static bool carve(const Plan* p, int64_t n_images, void* ws, size_t ws_bytes, Workspace* out) {
   const size_t chain = align256((size_t)chain_elems(p, n_images) * sizeof(float2));
   const size_t modes = align256((size_t)(n_images * p->n_modes_total) * sizeof(float2));
-  const size_t need = 2 * chain + 2 * modes;
+  const size_t need = 2 * chain + 2 * modes + grid32_bytes(p, n_images);
   if (need > 0 && (ws == nullptr || ws_bytes < need)) { set_error("workspace too small (see sc_workspace_bytes)"); return false; }
   char* base = static_cast<char*>(ws);
   out->buf[0] = reinterpret_cast<float2*>(base);
   out->buf[1] = reinterpret_cast<float2*>(base + chain);
   out->modes[0] = reinterpret_cast<float2*>(base + 2 * chain);
   out->modes[1] = reinterpret_cast<float2*>(base + 2 * chain + modes);
+  out->grid32 = p->grid16 ? reinterpret_cast<float*>(base + 2 * chain + 2 * modes) : nullptr;
   return true;
 }
 
@@ -286,38 +299,39 @@ static bool synthesize_generic(const Plan* p, const float2* modes_in, int64_t n_
                                 lead, n_channels > 0 ? n_channels : 1, st);
 }
 
-static bool analyze(const Plan* p, const float* images, int64_t n_images, float2* modes_out, bool adjoint,
-                    float2* b0, float2* b1, cudaStream_t st, bool quad_major = false, const L2Prefetch* pf = nullptr) {
+static bool analyze32(const Plan* p, const float* images, int64_t n_images, float2* modes_out, bool adjoint,
+                      float2* b0, float2* b1, cudaStream_t st, bool quad_major, const L2Prefetch* pf, int storage) {
   if (n_images <= 0) return true;
-  if (quad_major) return fast_analyze(p, images, n_images, modes_out, adjoint, st, true, pf);   // (dense_chain_quad_major checked the shape)
+  if (quad_major) return fast_analyze(p, images, n_images, modes_out, adjoint, st, true, pf, storage);   // (dense_chain_quad_major checked the shape)
   // tensor maps and bulk copies need 16-byte aligned bases: an offset view (e.g. buf[1:].view(...)) takes the generic chain
   const bool aligned = ((reinterpret_cast<uintptr_t>(images) | reinterpret_cast<uintptr_t>(modes_out)) & 15u) == 0;
   if (p->fast_enabled && aligned && fast_can_analyze(p, adjoint)) {
     if (p->d == 2) {
       if (n_images % fast_tile_group(p, false, adjoint) == 0)
-        return fast_analyze(p, images, n_images, modes_out, adjoint, st, false, pf);
+        return fast_analyze(p, images, n_images, modes_out, adjoint, st, false, pf, storage);
     } else {   // d == 3: fused last two dims per (image, z) slice, then dim 0 on the truncated data
       const DimTables& Z = p->dim[0];
       const int64_t slices = n_images * (adjoint ? Z.M : Z.N);
       if (slices % fast_tile_group(p, false, adjoint) == 0) {
-        if (!fast_analyze(p, images, slices, b0, adjoint, st)) return false;
+        if (!fast_analyze(p, images, slices, b0, adjoint, st, false, nullptr, storage)) return false;
         const int64_t inner = (int64_t)p->dim[1].k * p->dim[2].k;
         return launch_complex_table_gemm(adjoint ? Z.d_SH : Z.d_A, b0, modes_out, n_images, Z.k, adjoint ? Z.M : Z.N, (int)inner, st);
       }
     }
   }
+  if (storage != 0) { set_error("analyze: 16-bit images reached the float-only chain"); return false; }
   return analyze_generic(p, images, n_images, modes_out, adjoint, b0, b1, st);
 }
 
-static bool synthesize(const Plan* p, const float2* modes_in, int64_t n_images, int n_channels, const float* bias,
-                       float* images_out, bool adjoint, float2* b0, float2* b1, cudaStream_t st, bool quad_major = false) {
+static bool synthesize32(const Plan* p, const float2* modes_in, int64_t n_images, int n_channels, const float* bias,
+                         float* images_out, bool adjoint, float2* b0, float2* b1, cudaStream_t st, bool quad_major, int storage) {
   if (n_images <= 0) return true;
-  if (quad_major) return fast_synthesize(p, modes_in, n_images, n_channels, bias, images_out, adjoint, 1, st, true);
+  if (quad_major) return fast_synthesize(p, modes_in, n_images, n_channels, bias, images_out, adjoint, 1, st, true, storage);
   const bool aligned = ((reinterpret_cast<uintptr_t>(images_out) | reinterpret_cast<uintptr_t>(modes_in)) & 15u) == 0;
   if (p->fast_enabled && aligned && fast_can_synthesize(p, adjoint)) {
     if (p->d == 2) {
       if (n_images % fast_tile_group(p, true, adjoint) == 0)
-        return fast_synthesize(p, modes_in, n_images, n_channels, bias, images_out, adjoint, 1, st);
+        return fast_synthesize(p, modes_in, n_images, n_channels, bias, images_out, adjoint, 1, st, false, storage);
     } else {
       const DimTables& Z = p->dim[0];
       const int P0 = adjoint ? Z.N : Z.M;
@@ -325,11 +339,59 @@ static bool synthesize(const Plan* p, const float2* modes_in, int64_t n_images, 
       if (slices % fast_tile_group(p, true, adjoint) == 0) {
         const int64_t inner = (int64_t)p->dim[1].k * p->dim[2].k;
         if (!launch_complex_table_gemm(adjoint ? Z.d_AH : Z.d_S, modes_in, b0, n_images, P0, Z.k, (int)inner, st)) return false;
-        return fast_synthesize(p, b0, slices, n_channels, bias, images_out, adjoint, P0, st);
+        return fast_synthesize(p, b0, slices, n_channels, bias, images_out, adjoint, P0, st, false, storage);
       }
     }
   }
+  if (storage != 0) { set_error("synthesize: 16-bit images reached the float-only chain"); return false; }
   return synthesize_generic(p, modes_in, n_images, n_channels, bias, images_out, adjoint, b0, b1, st);
+}
+
+// Whether analyze32 / synthesize32 take the fused tensor-core kernels for this call (the same tests they make, in the same order).
+static bool fused_analysis_taken(const Plan* p, const void* images, int64_t n_images, const void* modes_out, bool adjoint, bool quad_major) {
+  if (quad_major) return true;
+  const bool aligned = ((reinterpret_cast<uintptr_t>(images) | reinterpret_cast<uintptr_t>(modes_out)) & 15u) == 0;
+  if (!(p->fast_enabled && aligned && fast_can_analyze(p, adjoint))) return false;
+  const int64_t units = p->d == 2 ? n_images : n_images * (adjoint ? p->dim[0].M : p->dim[0].N);
+  return (p->d == 2 || p->d == 3) && units % fast_tile_group(p, false, adjoint) == 0;
+}
+
+static bool fused_synthesis_taken(const Plan* p, const void* modes_in, int64_t n_images, const void* images_out, bool adjoint, bool quad_major) {
+  if (quad_major) return true;
+  const bool aligned = ((reinterpret_cast<uintptr_t>(images_out) | reinterpret_cast<uintptr_t>(modes_in)) & 15u) == 0;
+  if (!(p->fast_enabled && aligned && fast_can_synthesize(p, adjoint))) return false;
+  const int64_t units = p->d == 2 ? n_images : n_images * (adjoint ? p->dim[0].N : p->dim[0].M);
+  return (p->d == 2 || p->d == 3) && units % fast_tile_group(p, true, adjoint) == 0;
+}
+
+// The storage type of the images on `grid` is decided here and nowhere else.  With 16-bit storage the fused tensor-core kernels
+// read x / write dx at 16 bits themselves (k_fused_analysis2 widens each element before its hi / lo split, k_fused_synthesis
+// rounds in its epilogue); every other chain -- a misaligned view, the rows and generic kernels, the first-generation analysis --
+// runs on an fp32 copy in the workspace (widened exactly before the analysis, rounded to nearest even after the adjoint synthesis).
+// Either way the arithmetic is that of the float path on the widened input.  y / gy are always float.
+static bool analyze(const Plan* p, const float* images, int64_t n_images, float2* modes_out, bool adjoint, const Workspace& w,
+                    cudaStream_t st, bool quad_major = false, const L2Prefetch* pf = nullptr) {
+  if (n_images <= 0) return true;
+  if (p->grid16 && !adjoint) {
+    if (((reinterpret_cast<uintptr_t>(images) & 15u) == 0) && fast_analysis_reads_16bit(p) &&
+        fused_analysis_taken(p, images, n_images, modes_out, adjoint, quad_major))
+      return analyze32(p, images, n_images, modes_out, adjoint, w.buf[0], w.buf[1], st, quad_major, pf, p->grid16);
+    if (!launch_grid_convert(p->grid16, images, w.grid32, n_images * p->grid_points, false, st)) return false;
+    images = w.grid32;
+  }
+  return analyze32(p, images, n_images, modes_out, adjoint, w.buf[0], w.buf[1], st, quad_major, pf, 0);
+}
+
+static bool synthesize(const Plan* p, const float2* modes_in, int64_t n_images, int n_channels, const float* bias,
+                       float* images_out, bool adjoint, const Workspace& w, cudaStream_t st, bool quad_major = false) {
+  if (n_images <= 0) return true;
+  if (p->grid16 && adjoint) {
+    if (((reinterpret_cast<uintptr_t>(images_out) & 15u) == 0) && fused_synthesis_taken(p, modes_in, n_images, images_out, adjoint, quad_major))
+      return synthesize32(p, modes_in, n_images, n_channels, bias, images_out, adjoint, w.buf[0], w.buf[1], st, quad_major, p->grid16);
+    return synthesize32(p, modes_in, n_images, n_channels, bias, w.grid32, adjoint, w.buf[0], w.buf[1], st, quad_major, 0) &&
+           launch_grid_convert(p->grid16, w.grid32, images_out, n_images * p->grid_points, true, st);
+  }
+  return synthesize32(p, modes_in, n_images, n_channels, bias, images_out, adjoint, w.buf[0], w.buf[1], st, quad_major, 0);
 }
 
 // `chained`: the call is part of sc_forward_dense / sc_backward_dense, i.e. the kernel launched just before on the stream is
@@ -554,7 +616,7 @@ size_t sc_workspace_bytes(const sc_plan* plan, int64_t n_images) {
   const Plan* p = reinterpret_cast<const Plan*>(plan);
   if (p == nullptr || n_images <= 0) return 0;
   return 2 * align256((size_t)chain_elems(p, n_images) * sizeof(float2)) +
-         2 * align256((size_t)(n_images * p->n_modes_total) * sizeof(float2));
+         2 * align256((size_t)(n_images * p->n_modes_total) * sizeof(float2)) + grid32_bytes(p, n_images);
 }
 
 int sc_plan_set_fast_path(sc_plan* plan, int enable) {
@@ -586,8 +648,7 @@ int sc_analyze(const sc_plan* plan, const float* images, int64_t n_images, sc_co
   SC_REQUIRE(p != nullptr && images != nullptr && modes_out != nullptr, "sc_analyze: null argument");
   Workspace w{};
   SC_TRY(carve(p, n_images, workspace, workspace_bytes, &w));
-  SC_TRY(analyze(p, images, n_images, reinterpret_cast<float2*>(modes_out), adjoint != 0, w.buf[0], w.buf[1],
-                 static_cast<cudaStream_t>(stream)));
+  SC_TRY(analyze(p, images, n_images, reinterpret_cast<float2*>(modes_out), adjoint != 0, w, static_cast<cudaStream_t>(stream)));
   return 0;
 }
 
@@ -601,7 +662,7 @@ int sc_synthesize(const sc_plan* plan, const sc_complex* modes_in, int64_t n_ima
   Workspace w{};
   SC_TRY(carve(p, n_images, workspace, workspace_bytes, &w));
   SC_TRY(synthesize(p, reinterpret_cast<const float2*>(modes_in), n_images, n_channels, bias, images_out,
-                    adjoint != 0, w.buf[0], w.buf[1], static_cast<cudaStream_t>(stream)));
+                    adjoint != 0, w, static_cast<cudaStream_t>(stream)));
   return 0;
 }
 
@@ -652,14 +713,14 @@ int sc_forward_dense(const sc_plan* plan, const float* x, const sc_complex* weig
   // without a place to report it the saved modes stay in the standard layout
   const bool qm = saved_layout_out != nullptr && dense_chain_quad_major(p, batch, in_channels, out_channels, weight) &&
                   (reinterpret_cast<uintptr_t>(xm_saved) & 31u) == 0 &&
-                  ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 15u) == 0;
+                  (((p->grid16 ? 0 : reinterpret_cast<uintptr_t>(x)) | reinterpret_cast<uintptr_t>(y)) & 15u) == 0;   // 16-bit x: read from the workspace copy
   if (saved_layout_out != nullptr) *saved_layout_out = qm ? SC_MODES_QUAD_MAJOR : SC_MODES_STANDARD;
   // the forward contraction reads the whole weight right after the analysis: let the analysis launch pull it into L2
   L2Prefetch pf;
   pf.ptr[0] = weight; pf.bytes[0] = (unsigned long long)in_channels * out_channels * p->weight_elems_per_io * sizeof(float2);
-  SC_TRY(analyze(p, x, (int64_t)batch * in_channels, xm, false, w.buf[0], w.buf[1], st, qm, &pf));
+  SC_TRY(analyze(p, x, (int64_t)batch * in_channels, xm, false, w, st, qm, &pf));
   SC_TRY(contract_fwd(p, xm, reinterpret_cast<const float2*>(weight), ym, batch, in_channels, out_channels, st, true, qm, qm));
-  SC_TRY(synthesize(p, ym, (int64_t)batch * out_channels, out_channels, bias, y, false, w.buf[0], w.buf[1], st, qm));
+  SC_TRY(synthesize(p, ym, (int64_t)batch * out_channels, out_channels, bias, y, false, w, st, qm));
   return 0;
 }
 
@@ -681,20 +742,20 @@ int sc_backward_dense(const sc_plan* plan, const float* gy, const sc_complex* we
   // with the standalone kernel, which wants the standard layout)
   const bool g_qm = dense_chain_quad_major(p, batch, in_channels, out_channels, weight) && (dbias == nullptr || dweight != nullptr) &&
                     (dweight == nullptr || (reinterpret_cast<uintptr_t>(dweight) & 31u) == 0) &&
-                    ((reinterpret_cast<uintptr_t>(gy) | reinterpret_cast<uintptr_t>(dx)) & 15u) == 0;
+                    ((reinterpret_cast<uintptr_t>(gy) | (p->grid16 ? 0 : reinterpret_cast<uintptr_t>(dx))) & 15u) == 0;
   SC_REQUIRE(!x_qm || p->fast != nullptr, "sc_backward_dense: quad-major saved modes without the tensor-core path");
   // the two backward contractions read the saved modes and the weight: the gy analysis pulls both into L2
   L2Prefetch pf;
   if (dweight != nullptr) { pf.ptr[0] = xm_saved; pf.bytes[0] = (unsigned long long)batch * in_channels * p->n_modes_total * sizeof(float2); }
   if (dx != nullptr) { pf.ptr[1] = weight; pf.bytes[1] = (unsigned long long)in_channels * out_channels * p->weight_elems_per_io * sizeof(float2); }
-  SC_TRY(analyze(p, gy, (int64_t)batch * out_channels, gm, true, w.buf[0], w.buf[1], st, g_qm, &pf));
+  SC_TRY(analyze(p, gy, (int64_t)batch * out_channels, gm, true, w, st, g_qm, &pf));
   SC_TRY(contract_bwd(p, reinterpret_cast<const float2*>(xm_saved), gm, reinterpret_cast<const float2*>(weight), dxm,
                       reinterpret_cast<float2*>(dweight), dbias, batch, in_channels, out_channels, st, true, x_qm, g_qm,
                       static_cast<cudaEvent_t>(grads_ready)));
   if (dx != nullptr) {
     // with a collective running on the caller's side stream (grads_ready given), the dx synthesis leaves SMs free for it
     fast_set_reserve(grads_ready != nullptr);
-    const bool ok = synthesize(p, dxm, (int64_t)batch * in_channels, 0, nullptr, dx, true, w.buf[0], w.buf[1], st, g_qm);
+    const bool ok = synthesize(p, dxm, (int64_t)batch * in_channels, 0, nullptr, dx, true, w, st, g_qm);
     fast_set_reserve(false);
     SC_TRY(ok);
   }
@@ -794,7 +855,7 @@ int sc_forward_tucker(const sc_plan* plan, const sc_plan* plan_kept, const float
   float2* sv = reinterpret_cast<float2*>(saved);
   float2 *xm = sv + t.off_xm(), *t1 = sv + t.off_t1(), *t2 = sv + t.off_t2(), *wc = sv + t.off_wc();
   float2* ym = w.modes[0];
-  SC_TRY(analyze(p, x, (int64_t)t.B * t.Ci, xm, false, w.buf[0], w.buf[1], st));
+  SC_TRY(analyze(p, x, (int64_t)t.B * t.Ci, xm, false, w, st));
   // expand the core along the mode axes, last axis first: A_d = core, A_j = U_j x_j A_{j+1}   (A_0 = wc)
   const float2* cur = reinterpret_cast<const float2*>(core);
   for (int j = t.d - 1; j >= 0; --j) {
@@ -807,7 +868,7 @@ int sc_forward_tucker(const sc_plan* plan, const sc_plan* plan_kept, const float
   SC_TRY(launch_complex_table_gemm_strided(reinterpret_cast<const float2*>(u_in), 1, t.rf, false, xm, t1, t.B, t.rf, t.Ci, (int)t.M, st));
   SC_TRY(contract_fwd(pk, t1, wc, t2, t.B, t.rf, t.rg, st, false));
   SC_TRY(launch_complex_table_gemm_strided(reinterpret_cast<const float2*>(u_out), t.rg, 1, false, t2, ym, t.B, t.Co, t.rg, (int)t.M, st));
-  SC_TRY(synthesize(p, ym, (int64_t)t.B * t.Co, t.Co, bias, y, false, w.buf[0], w.buf[1], st));
+  SC_TRY(synthesize(p, ym, (int64_t)t.B * t.Co, t.Co, bias, y, false, w, st));
   return 0;
 }
 
@@ -834,7 +895,7 @@ int sc_backward_tucker(const sc_plan* plan, const sc_plan* plan_kept, const floa
   const float2 *xm = sv + t.off_xm(), *t1 = sv + t.off_t1(), *t2 = sv + t.off_t2(), *wc = sv + t.off_wc();
   float2* gm = w.modes[0];
   float2* dxm = w.modes[1];
-  SC_TRY(analyze(p, gy, (int64_t)t.B * t.Co, gm, true, w.buf[0], w.buf[1], st));
+  SC_TRY(analyze(p, gy, (int64_t)t.B * t.Co, gm, true, w, st));
   if (dbias != nullptr) SC_TRY(launch_bias_grad(gm, dbias, t.B, t.Co, t.M, p->dc_slot, (float)(1.0 / p->s_inv), st));
   // out side: g2 = U_out^H gm,  dU_out[o, g] = sum conj(t2[b, g, m]) gm[b, o, m]
   SC_TRY(launch_complex_table_gemm_strided(reinterpret_cast<const float2*>(u_out), 1, t.rg, true, gm, a.g2, t.B, t.rg, t.Co, (int)t.M, st));
@@ -844,7 +905,7 @@ int sc_backward_tucker(const sc_plan* plan, const sc_plan* plan_kept, const floa
   // in side
   SC_TRY(launch_pair_reduce(xm, a.g1, reinterpret_cast<float2*>(d_u_in), t.rf, 1, t.B, t.Ci, t.rf, (int)t.M, st));
   SC_TRY(launch_complex_table_gemm_strided(reinterpret_cast<const float2*>(u_in), t.rf, 1, true, a.g1, dxm, t.B, t.Ci, t.rf, (int)t.M, st));
-  SC_TRY(synthesize(p, dxm, (int64_t)t.B * t.Ci, 0, nullptr, dx, true, w.buf[0], w.buf[1], st));
+  SC_TRY(synthesize(p, dxm, (int64_t)t.B * t.Ci, 0, nullptr, dx, true, w, st));
   // mode factors and core: undo the expansion chain, first axis first
   const float2* d_a = a.dwc;
   for (int j = 0; j < t.d; ++j) {
@@ -968,15 +1029,15 @@ void ch_log(int op, A... a) {
   (t_chain_log->push_back(ch_word(a)), ...);
 }
 
-bool ch_analyze(const Plan* p, const float* images, int64_t n_images, float2* modes_out, bool adjoint, float2* b0, float2* b1,
+bool ch_analyze(const Plan* p, const float* images, int64_t n_images, float2* modes_out, bool adjoint, const Workspace& w,
                 cudaStream_t st) {
   if (t_chain_log != nullptr) { ch_log(CH_ANALYZE, images, n_images, modes_out, adjoint); return true; }
-  return analyze(p, images, n_images, modes_out, adjoint, b0, b1, st);
+  return analyze(p, images, n_images, modes_out, adjoint, w, st);
 }
 bool ch_synthesize(const Plan* p, const float2* modes_in, int64_t n_images, int n_channels, const float* bias, float* images_out,
-                   bool adjoint, float2* b0, float2* b1, cudaStream_t st) {
+                   bool adjoint, const Workspace& w, cudaStream_t st) {
   if (t_chain_log != nullptr) { ch_log(CH_SYNTHESIZE, modes_in, n_images, n_channels, bias, images_out, adjoint); return true; }
-  return synthesize(p, modes_in, n_images, n_channels, bias, images_out, adjoint, b0, b1, st);
+  return synthesize(p, modes_in, n_images, n_channels, bias, images_out, adjoint, w, st);
 }
 bool ch_table(const float2* T, int64_t sTp, int64_t sTq, bool conjT, const float2* in, float2* out, int64_t O, int P, int Q, int I,
               cudaStream_t st) {
@@ -1095,13 +1156,13 @@ int sc_forward_cp(const sc_plan* plan, const float* x, const sc_complex* lambda,
   float2* sv = reinterpret_cast<float2*>(saved);
   float2 *xm = sv, *t1 = sv + t.off_t1(), *t2 = sv + t.off_t2(), *scale = sv + t.off_scale();
   float2* ym = w.modes[0];
-  SC_TRY(ch_analyze(p, x, (int64_t)t.B * t.Ci, xm, false, w.buf[0], w.buf[1], st));
+  SC_TRY(ch_analyze(p, x, (int64_t)t.B * t.Ci, xm, false, w, st));
   SC_TRY(ch_cp_scale(u, k, t.d, reinterpret_cast<const float2*>(lambda), scale, t.R, t.M, st));
   // T[p = e, q = i] = U_in[i, e];  pointwise scale;  T[p = o, q = e] = U_out[o, e]
   SC_TRY(ch_table(reinterpret_cast<const float2*>(u_in), 1, t.R, false, xm, t1, t.B, t.R, t.Ci, (int)t.M, st));
   SC_TRY(ch_cp_apply(t1, scale, t2, false, t.B, (int64_t)t.R * t.M, st));
   SC_TRY(ch_table(reinterpret_cast<const float2*>(u_out), t.R, 1, false, t2, ym, t.B, t.Co, t.R, (int)t.M, st));
-  SC_TRY(ch_synthesize(p, ym, (int64_t)t.B * t.Co, t.Co, bias, y, false, w.buf[0], w.buf[1], st));
+  SC_TRY(ch_synthesize(p, ym, (int64_t)t.B * t.Co, t.Co, bias, y, false, w, st));
   return 0;
 }
 
@@ -1131,7 +1192,7 @@ int sc_backward_cp(const sc_plan* plan, const float* gy, const sc_complex* lambd
   float2* gm = w.modes[0];
   float2* dxm = w.modes[1];
   const int64_t per = (int64_t)t.R * t.M;
-  SC_TRY(ch_analyze(p, gy, (int64_t)t.B * t.Co, gm, true, w.buf[0], w.buf[1], st));
+  SC_TRY(ch_analyze(p, gy, (int64_t)t.B * t.Co, gm, true, w, st));
   if (dbias != nullptr) SC_TRY(ch_bias_grad(gm, dbias, t.B, t.Co, t.M, p->dc_slot, (float)(1.0 / p->s_inv), st));
   // out side: g2 = U_out^H gm,  dU_out[o, e] = sum conj(t2[b, e, m]) gm[b, o, m]
   SC_TRY(ch_table(reinterpret_cast<const float2*>(u_out), 1, t.R, true, gm, a.g2, t.B, t.R, t.Co, (int)t.M, st));
@@ -1142,7 +1203,7 @@ int sc_backward_cp(const sc_plan* plan, const float* gy, const sc_complex* lambd
   // in side
   SC_TRY(ch_pair(xm, a.g1, reinterpret_cast<float2*>(d_u_in), t.R, 1, t.B, t.Ci, t.R, (int)t.M, st));
   SC_TRY(ch_table(reinterpret_cast<const float2*>(u_in), t.R, 1, true, a.g1, dxm, t.B, t.Ci, t.R, (int)t.M, st));
-  SC_TRY(ch_synthesize(p, dxm, (int64_t)t.B * t.Ci, 0, nullptr, dx, true, w.buf[0], w.buf[1], st));
+  SC_TRY(ch_synthesize(p, dxm, (int64_t)t.B * t.Ci, 0, nullptr, dx, true, w, st));
   // lambda and the mode factors from dscale
   SC_TRY(ch_cp_factor_grad(u, k, t.d, lam, a.dscale, reinterpret_cast<float2*>(d_lambda), -1, t.R, t.M, st));
   for (int j = 0; j < t.d; ++j)
@@ -1234,7 +1295,7 @@ int sc_forward_tt(const sc_plan* plan, const sc_plan* plan_kept, const float* x,
   float2* sv = reinterpret_cast<float2*>(saved);
   float2 *xm = sv, *t1 = sv + t.off_t1(), *wc = sv + t.off_wc();
   float2* ym = w.modes[0];
-  SC_TRY(ch_analyze(p, x, (int64_t)t.B * t.Ci, xm, false, w.buf[0], w.buf[1], st));
+  SC_TRY(ch_analyze(p, x, (int64_t)t.B * t.Ci, xm, false, w, st));
   // A_{d-1} = cores[d-1] (r_{d-1}, k_{d-1});  A_j[(a, m_j), rest] = sum_b C_j[a, m_j, b] A_{j+1}[b, rest];  V = A_0 (r_0, M)
   const float2* cur = reinterpret_cast<const float2*>(cores[t.d - 1]);
   for (int j = t.d - 2; j >= 0; --j) {
@@ -1247,7 +1308,7 @@ int sc_forward_tt(const sc_plan* plan, const sc_plan* plan_kept, const float* x,
   SC_TRY(ch_table(reinterpret_cast<const float2*>(g1), t.r[0], 1, false, cur, wc, 1, t.r1 * t.Co, t.r[0], (int)t.M, st));
   SC_TRY(ch_table(reinterpret_cast<const float2*>(g0), 1, t.r1, false, xm, t1, t.B, t.r1, t.Ci, (int)t.M, st));
   SC_TRY(ch_contract_fwd(pk, t1, wc, ym, t.B, t.r1, t.Co, st));
-  SC_TRY(ch_synthesize(p, ym, (int64_t)t.B * t.Co, t.Co, bias, y, false, w.buf[0], w.buf[1], st));
+  SC_TRY(ch_synthesize(p, ym, (int64_t)t.B * t.Co, t.Co, bias, y, false, w, st));
   return 0;
 }
 
@@ -1273,14 +1334,14 @@ int sc_backward_tt(const sc_plan* plan, const sc_plan* plan_kept, const float* g
   const float2 *xm = sv, *t1 = sv + t.off_t1(), *wc = sv + t.off_wc();
   float2* gm = w.modes[0];
   float2* dxm = w.modes[1];
-  SC_TRY(ch_analyze(p, gy, (int64_t)t.B * t.Co, gm, true, w.buf[0], w.buf[1], st));
+  SC_TRY(ch_analyze(p, gy, (int64_t)t.B * t.Co, gm, true, w, st));
   if (dbias != nullptr) SC_TRY(ch_bias_grad(gm, dbias, t.B, t.Co, t.M, p->dc_slot, (float)(1.0 / p->s_inv), st));
   // the two mode GEMMs of the dense backward on the rank channels: g1 = d(t1), dwc = d(wc)
   SC_TRY(ch_contract_bwd(pk, t1, gm, wc, a.g1, a.dwc, t.B, t.r1, t.Co, st));
   // in side: dG0[0, i, r] = sum conj(xm[b, i, m]) g1[b, r, m];  dxm = g1 G0^H
   SC_TRY(ch_pair(xm, a.g1, reinterpret_cast<float2*>(d_g0), t.r1, 1, t.B, t.Ci, t.r1, (int)t.M, st));
   SC_TRY(ch_table(reinterpret_cast<const float2*>(g0), t.r1, 1, true, a.g1, dxm, t.B, t.Ci, t.r1, (int)t.M, st));
-  SC_TRY(ch_synthesize(p, dxm, (int64_t)t.B * t.Ci, 0, nullptr, dx, true, w.buf[0], w.buf[1], st));
+  SC_TRY(ch_synthesize(p, dxm, (int64_t)t.B * t.Ci, 0, nullptr, dx, true, w, st));
   // weight side: dG1[(r, o), s] = sum_m conj(V[s, m]) dwc[(r, o), m];  dV = G1^H dwc;  then undo the chain, first axis first
   const float2* v = t.d >= 2 ? sv + t.off_chain(0) : reinterpret_cast<const float2*>(cores[0]);
   SC_TRY(ch_pair(v, a.dwc, reinterpret_cast<float2*>(d_g1), 1, t.r[0], 1, t.r[0], t.r1 * t.Co, (int)t.M, st));

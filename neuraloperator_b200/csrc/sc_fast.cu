@@ -12,6 +12,7 @@
 #include <vector>
 
 #include "sc_fast.h"
+#include "sc_half.cuh"
 #include "sc_umma.cuh"
 
 namespace sc {
@@ -534,7 +535,10 @@ __global__ void __launch_bounds__(FA_THREADS, 1) k_fused_analysis(const AnaParam
 // =====================================================================================================
 constexpr int FA2_X_STAGES = 2, FA2_MAX_F32 = 6;
 
-template <int N1>
+// S: storage of x -- 0 float ([128 x 32 floats] boxes, two per slab), SC_FLAG_GRID_F16 / SC_FLAG_GRID_BF16 (one [128 x 64 elements]
+// box per slab: the same 128-byte rows and swizzle, half the bytes; the converters widen each element before the hi / lo split,
+// so the operands are bit for bit those of the float path on the widened input)
+template <int N1, int S>
 __global__ void __launch_bounds__(FA_THREADS, 1) k_fused_analysis2(const AnaParams P, const __grid_constant__ CUtensorMap x_map,
                                                                      const __grid_constant__ CUtensorMap qm_map) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -622,9 +626,11 @@ __global__ void __launch_bounds__(FA_THREADS, 1) k_fused_analysis2(const AnaPara
         }
         const int tile = (int)blockIdx.x + (idx / P.slabs) * (int)gridDim.x, slab = idx % P.slabs;
         // a slab = two [128 rows x 32 floats] boxes in the 128-byte swizzle: a thread can then read ITS ROW conflict-free
-        mbar_arrive_expect_tx(&bar_f32_full[sb], 32768u);
+        // (16-bit x: ONE [128 rows x 64 elements] box, same row length and swizzle)
+        constexpr int n_boxes = S == 0 ? 2 : 1;
+        mbar_arrive_expect_tx(&bar_f32_full[sb], (uint32_t)(n_boxes * 16384));
 #pragma unroll
-        for (int hb = 0; hb < 2; ++hb) {
+        for (int hb = 0; hb < n_boxes; ++hb) {
           if (P.l2_stream_hint) tma_load_2d_hint(f32_stage + sb * 32768 + hb * 16384, &x_map, &bar_f32_full[sb], slab * 64 + hb * 32, tile * 128, pol);
           else tma_load_2d(f32_stage + sb * 32768 + hb * 16384, &x_map, &bar_f32_full[sb], slab * 64 + hb * 32, tile * 128);
         }
@@ -640,7 +646,7 @@ __global__ void __launch_bounds__(FA_THREADS, 1) k_fused_analysis2(const AnaPara
     const int cw = warp - FA_LOADER_WARP0, q = warp & 3, hb = cw >> 2;
     const int row = 32 * q + lane;
     uint8_t* f32_stage = smem + P.off_f32;
-    const uint32_t my_row = (uint32_t)(hb * 16384 + row * 128);
+    const uint32_t my_row = (uint32_t)((S == 0 ? hb * 16384 : 0) + row * 128);
     const uint32_t sw = (uint32_t)(row & 7);
     const uint32_t tm_mine = tm_x + ((uint32_t)(32 * q) << 16) + (uint32_t)(16 * hb);
     const int total = n_local * P.slabs;
@@ -652,11 +658,22 @@ __global__ void __launch_bounds__(FA_THREADS, 1) k_fused_analysis2(const AnaPara
       if (warp == FA_LOADER_WARP0) SC_TRACE(P, 7, idx, 0);
       uint32_t hi[16], lo[16];
       const uint8_t* fsrc = f32_stage + sb * 32768 + my_row;
+      if constexpr (S == 0) {
 #pragma unroll
-      for (int c = 0; c < 8; ++c) {            // 16-byte chunk c of the row sits at chunk position c ^ (row & 7)
-        const float4 v = *reinterpret_cast<const float4*>(fsrc + ((c ^ sw) << 4));
-        split2_bf16(v.x, v.y, hi[2 * c], lo[2 * c]);
-        split2_bf16(v.z, v.w, hi[2 * c + 1], lo[2 * c + 1]);
+        for (int c = 0; c < 8; ++c) {            // 16-byte chunk c of the row sits at chunk position c ^ (row & 7)
+          const float4 v = *reinterpret_cast<const float4*>(fsrc + ((c ^ sw) << 4));
+          split2_bf16(v.x, v.y, hi[2 * c], lo[2 * c]);
+          split2_bf16(v.z, v.w, hi[2 * c + 1], lo[2 * c + 1]);
+        }
+      } else {
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {            // this warp's half of the row: 16-byte chunks 4 hb .. 4 hb + 3, 8 elements each
+          const uint4 v = *reinterpret_cast<const uint4*>(fsrc + (((4 * hb + c) ^ sw) << 4));
+          const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+          for (int e = 0; e < 4; ++e)
+            split2_bf16(g16_load<S>((uint16_t)(w[e] & 0xffffu)), g16_load<S>((uint16_t)(w[e] >> 16)), hi[4 * c + e], lo[4 * c + e]);
+        }
       }
       __syncwarp();
       if (lane == 0) mbar_arrive(&bar_f32_empty[sb]);   // this warp has consumed its pieces of the staging buffer
@@ -885,7 +902,9 @@ struct SynParams {
   long long* trace;        // debug timeline of CTA 0 (SC_TRACE_FILE), else nullptr
 };
 
-template <int N1>
+// S: storage of the output -- 0 float, SC_FLAG_GRID_F16 / SC_FLAG_GRID_BF16 (only the adjoint synthesis, dx, is launched so): the
+// epilogue rounds to nearest even and stores [32 rows x 32 elements] boxes of 64-byte rows in the 64-byte swizzle
+template <int N1, int S>
 __global__ void __launch_bounds__(FS_THREADS, 1) k_fused_synthesis(const SynParams P, const __grid_constant__ CUtensorMap out_map) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -1123,14 +1142,26 @@ __global__ void __launch_bounds__(FS_THREADS, 1) k_fused_synthesis(const SynPara
         if (lane == 0) bulk_wait_read();            // the previous store of this warp has finished reading the box
         __syncwarp();
         tmem_ld_wait();
+        if constexpr (S == 0) {
 #pragma unroll
-        for (int u = 0; u < 2; ++u)
+          for (int u = 0; u < 2; ++u)
 #pragma unroll
-          for (int e = 0; e < 16; e += 4) {
-            const int ch = (16 * u + e) >> 2;        // 16-byte chunk index within the 128-byte row
-            *reinterpret_cast<float4*>(box + lane * 128 + (((ch ^ lane) & 7) << 4)) =
-                make_float4(t[u][e] + b, t[u][e + 1] + b, t[u][e + 2] + b, t[u][e + 3] + b);
-          }
+            for (int e = 0; e < 16; e += 4) {
+              const int ch = (16 * u + e) >> 2;        // 16-byte chunk index within the 128-byte row
+              *reinterpret_cast<float4*>(box + lane * 128 + (((ch ^ lane) & 7) << 4)) =
+                  make_float4(t[u][e] + b, t[u][e + 1] + b, t[u][e + 2] + b, t[u][e + 3] + b);
+            }
+        } else {
+#pragma unroll
+          for (int u = 0; u < 2; ++u)
+#pragma unroll
+            for (int e = 0; e < 16; e += 8) {
+              const int ch = (16 * u + e) >> 3;        // 16-byte chunk (8 elements) within the 64-byte row; 64-byte swizzle
+              *reinterpret_cast<uint4*>(box + lane * 64 + (((ch ^ (lane >> 1)) & 3) << 4)) =
+                  make_uint4(g16_pack2<S>(t[u][e] + b, t[u][e + 1] + b), g16_pack2<S>(t[u][e + 2] + b, t[u][e + 3] + b),
+                             g16_pack2<S>(t[u][e + 4] + b, t[u][e + 5] + b), g16_pack2<S>(t[u][e + 6] + b, t[u][e + 7] + b));
+            }
+        }
         fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) {
@@ -2225,8 +2256,11 @@ static bool thread_has_context() {
 }
 
 static bool make_swizzled_box_map(CUtensorMap* map, const float* base, uint64_t rows, uint64_t W);
-// kind 0: x slab loads, kind 1: image row-tile stores, kind 2: x loads as 128-byte-swizzled [128 x 32] boxes (k_fused_analysis2)
-static bool cached_map(const Plan* p, int kind, const void* base, uint64_t rows, uint64_t W, CUtensorMap* out) {
+static bool make_16bit_map(CUtensorMap* map, const void* base, uint64_t rows, uint64_t W, int storage, bool store);
+// kind 0: x slab loads, kind 1: image row-tile stores, kind 2: x loads as 128-byte-swizzled [128 x 32] boxes (k_fused_analysis2),
+// kinds 3 / 4: the 16-bit x loads / dx stores of make_16bit_map, with storage = SC_FLAG_GRID_F16 / SC_FLAG_GRID_BF16
+static bool cached_map(const Plan* p, int kind, const void* base, uint64_t rows, uint64_t W, CUtensorMap* out, int storage = 0) {
+  if (storage != 0) kind += 8 * storage;   // distinct cache keys per element type
   FastTables* f = p->fast;
   std::lock_guard<std::mutex> lock(f->map_mutex);
   for (const TensorMapCacheEntry& e : f->map_cache)
@@ -2238,7 +2272,9 @@ static bool cached_map(const Plan* p, int kind, const void* base, uint64_t rows,
   // buffers from the graph's private pool, i.e. cache misses), and a capturing thread always has its context.
   if (!thread_has_context()) cudaFree(nullptr);
   TensorMapCacheEntry e{base, rows, W, kind, {}};
-  const bool ok = kind == 0 ? make_slab_load_map(&e.map, static_cast<const float*>(base), rows, W)
+  const int base_kind = kind % 8;
+  const bool ok = storage != 0 ? make_16bit_map(&e.map, base, rows, W, storage, base_kind == 4)
+                  : kind == 0 ? make_slab_load_map(&e.map, static_cast<const float*>(base), rows, W)
                   : kind == 2 ? make_swizzled_box_map(&e.map, static_cast<const float*>(base), rows, W)
                               : make_row_tile_map(&e.map, static_cast<float*>(const_cast<void*>(base)), rows, W);
   if (!ok) return false;
@@ -2535,6 +2571,23 @@ static bool make_slab_load_map(CUtensorMap* map, const float* base, uint64_t row
   return true;
 }
 
+// 16-bit image matrix [rows x W] (row-major): kind 3 = x loads, boxes [128 rows x 64 elements] in the 128-byte swizzle
+// (k_fused_analysis2); kind 4 = dx stores, boxes [32 rows x 32 elements] in the 64-byte swizzle (k_fused_synthesis)
+static bool make_16bit_map(CUtensorMap* map, const void* base, uint64_t rows, uint64_t W, int storage, bool store) {
+  EncodeTiledFn enc = tensor_map_encoder();
+  if (enc == nullptr) { set_error("cuTensorMapEncodeTiled entry point not available"); return false; }
+  const cuuint64_t dims[2] = {W, rows};
+  const cuuint64_t strides[1] = {W * 2};
+  const cuuint32_t box[2] = {store ? 32u : 64u, store ? 32u : 128u};
+  const cuuint32_t estr[2] = {1, 1};
+  const CUresult r = enc(map, storage == SC_FLAG_GRID_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2,
+                         const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                         store ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B,
+                         store ? CU_TENSOR_MAP_L2_PROMOTION_NONE : CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled (16-bit images) failed: CUresult " + std::to_string((int)r)); return false; }
+  return true;
+}
+
 // 3-D view {contiguous floats, second index, quads} of a quad-major tensor: one request per 1 KB row of the box
 static bool cached_wide_map(const Plan* p, const float2* base, uint64_t inner_floats, uint64_t n_second, uint64_t nq, uint64_t stride_second_bytes,
                             uint64_t stride_quad_bytes, uint32_t box_inner, uint32_t box_second, CUtensorMap* out, uint32_t box_quads) {
@@ -2677,8 +2730,15 @@ static void trace_end(long long* d, const char* what) {
   fclose(f);
 }
 
+static bool ana2_enabled() {
+  static const bool on = [] { const char* e = getenv("SC_ANA2"); return e == nullptr || atoi(e) != 0; }();   // =0: first generation (A/B runs)
+  return on;
+}
+
+bool fast_analysis_reads_16bit(const Plan* p) { return p->fast != nullptr && p->fast->ana[0].v2_ok && ana2_enabled(); }
+
 bool fast_analyze(const Plan* p, const float* images, int64_t n_images, float2* modes_out, bool adjoint, cudaStream_t st,
-                  bool quad_major, const L2Prefetch* pf) {
+                  bool quad_major, const L2Prefetch* pf, int storage) {
   const FusedAnalysisTables& t = p->fast->ana[adjoint ? 1 : 0];
   if (quad_major && ((t.KY * t.KX) % 4 != 0 || (reinterpret_cast<uintptr_t>(modes_out) & 31u) != 0)) {
     set_error("fast_analyze: the quad-major layout needs a mode count that is a multiple of 4 and a 32-byte aligned buffer");
@@ -2704,11 +2764,11 @@ bool fast_analyze(const Plan* p, const float* images, int64_t n_images, float2* 
   P.trace = trace_begin();
   const int grid = persistent_grid(p, P.n_tiles);
   CUtensorMap x_map;
-  static const bool ana2_on = [] { const char* e = getenv("SC_ANA2"); return e == nullptr || atoi(e) != 0; }();   // =0: first generation (A/B runs)
-  if (t.v2_ok && ana2_on) {
+  if (storage != 0 && (adjoint || !fast_analysis_reads_16bit(p))) { set_error("fast_analyze: 16-bit images need k_fused_analysis2"); return false; }
+  if (t.v2_ok && ana2_enabled()) {
     P.n_stages = t.v2_stages; P.tmem_cols = 512;
     P.off_f32 = 0; P.off_ring = 0; P.off_b1 = t.v2_off_b1; P.off_a2 = t.v2_off_b2; P.off_b2 = t.v2_off_b2; P.off_scratch = t.v2_off_scratch;
-    if (!cached_map(p, 2, images, (uint64_t)P.n_tiles * 128, (uint64_t)t.W, &x_map)) return false;
+    if (!cached_map(p, storage ? 3 : 2, images, (uint64_t)P.n_tiles * 128, (uint64_t)t.W, &x_map, storage)) return false;
     CUtensorMap qm_map = x_map;   // (placeholder when unused)
     static const bool qm_tma_on = [] { const char* e = getenv("SC_QM_TMA"); return e == nullptr || atoi(e) != 0; }();   // =0: store loop (A/B runs)
     if (quad_major && qm_tma_on && t.G == 1 && P.Mt / 4 <= 256 && ((P.off_scratch + P.stage_off) % 128u) == 0 && (P.Mt * 8) % 128 == 0) {
@@ -2718,17 +2778,24 @@ bool fast_analyze(const Plan* p, const float* images, int64_t n_images, float2* 
       P.qm_tma = 1;
     }
     switch (t.N1) {
-#define SC_FA2_CASE(N)                                                                                           \
-  case N: {                                                                                                      \
+#define SC_FA2_LAUNCH(N, S)                                                                                      \
+  {                                                                                                              \
     static SmemOptIn opt_in;                                                                                     \
-    if (!ensure_dynamic_smem((const void*)k_fused_analysis2<N>, opt_in, p->device, t.v2_smem_bytes,              \
+    if (!ensure_dynamic_smem((const void*)k_fused_analysis2<N, S>, opt_in, p->device, t.v2_smem_bytes,           \
                              "cudaFuncSetAttribute(k_fused_analysis2)")) return false;                          \
-    { void* args[] = {(void*)&P, (void*)&x_map, (void*)&qm_map};                                              \
-      if (!cuda_ok(launch_pdl((const void*)k_fused_analysis2<N>, dim3(grid), dim3(FA_THREADS), t.v2_smem_bytes, st, args), \
-                   "k_fused_analysis2 launch")) return false; }                                             \
-  } break;
+    void* args[] = {(void*)&P, (void*)&x_map, (void*)&qm_map};                                                 \
+    if (!cuda_ok(launch_pdl((const void*)k_fused_analysis2<N, S>, dim3(grid), dim3(FA_THREADS), t.v2_smem_bytes, st, args), \
+                 "k_fused_analysis2 launch")) return false;                                                     \
+  }
+#define SC_FA2_CASE(N)                                                                                           \
+  case N:                                                                                                        \
+    if (storage == SC_FLAG_GRID_F16) SC_FA2_LAUNCH(N, SC_FLAG_GRID_F16)                                          \
+    else if (storage == SC_FLAG_GRID_BF16) SC_FA2_LAUNCH(N, SC_FLAG_GRID_BF16)                                   \
+    else SC_FA2_LAUNCH(N, 0)                                                                                     \
+    break;
       SC_FA2_CASE(16) SC_FA2_CASE(32) SC_FA2_CASE(48)
 #undef SC_FA2_CASE
+#undef SC_FA2_LAUNCH
       default: set_error("fast_analyze: unsupported N1"); return false;
     }
     count_launch();
@@ -2756,8 +2823,9 @@ bool fast_analyze(const Plan* p, const float* images, int64_t n_images, float2* 
 }
 
 bool fast_synthesize(const Plan* p, const float2* modes_in, int64_t n_images, int n_channels, const float* bias,
-                     float* images_out, bool adjoint, int slices_per_image, cudaStream_t st, bool quad_major) {
+                     float* images_out, bool adjoint, int slices_per_image, cudaStream_t st, bool quad_major, int storage) {
   const FusedSynthesisTables& t = p->fast->syn[adjoint ? 1 : 0];
+  if (storage != 0 && (!adjoint || bias != nullptr)) { set_error("fast_synthesize: 16-bit output is the adjoint synthesis (dx) only"); return false; }
   if (quad_major && (t.KY * t.KX) % 4 != 0) { set_error("fast_synthesize: the quad-major layout needs a mode count that is a multiple of 4"); return false; }
   if (n_images % t.G != 0) { set_error("fast_synthesize: image count not a multiple of the tile group"); return false; }
   SynParams P{};
@@ -2772,19 +2840,26 @@ bool fast_synthesize(const Plan* p, const float2* modes_in, int64_t n_images, in
   P.trace = trace_begin();
   const int grid = persistent_grid(p, P.n_tiles);
   CUtensorMap out_map;
-  if (!cached_map(p, 1, images_out, (uint64_t)P.n_tiles * 128, (uint64_t)t.W, &out_map)) return false;
+  if (!cached_map(p, storage ? 4 : 1, images_out, (uint64_t)P.n_tiles * 128, (uint64_t)t.W, &out_map, storage)) return false;
   switch (t.N1) {
-#define SC_FS_CASE(N)                                                                                            \
-  case N: {                                                                                                      \
+#define SC_FS_LAUNCH(N, S)                                                                                       \
+  {                                                                                                              \
     static SmemOptIn opt_in;                                                                                     \
-    if (!ensure_dynamic_smem((const void*)k_fused_synthesis<N>, opt_in, p->device, t.smem_bytes,                 \
+    if (!ensure_dynamic_smem((const void*)k_fused_synthesis<N, S>, opt_in, p->device, t.smem_bytes,              \
                              "cudaFuncSetAttribute(k_fused_synthesis)")) return false;                          \
-    { void* args[] = {(void*)&P, (void*)&out_map};                                                             \
-      if (!cuda_ok(launch_pdl((const void*)k_fused_synthesis<N>, dim3(grid), dim3(FS_THREADS), t.smem_bytes, st, args), \
-                   "k_fused_synthesis launch")) return false; }                                             \
-  } break;
+    void* args[] = {(void*)&P, (void*)&out_map};                                                               \
+    if (!cuda_ok(launch_pdl((const void*)k_fused_synthesis<N, S>, dim3(grid), dim3(FS_THREADS), t.smem_bytes, st, args), \
+                 "k_fused_synthesis launch")) return false;                                                     \
+  }
+#define SC_FS_CASE(N)                                                                                            \
+  case N:                                                                                                        \
+    if (storage == SC_FLAG_GRID_F16) SC_FS_LAUNCH(N, SC_FLAG_GRID_F16)                                           \
+    else if (storage == SC_FLAG_GRID_BF16) SC_FS_LAUNCH(N, SC_FLAG_GRID_BF16)                                    \
+    else SC_FS_LAUNCH(N, 0)                                                                                      \
+    break;
     SC_FS_CASE(16) SC_FS_CASE(32) SC_FS_CASE(48) SC_FS_CASE(64)
 #undef SC_FS_CASE
+#undef SC_FS_LAUNCH
     default: set_error("fast_synthesize: unsupported N1"); return false;
   }
   count_launch();

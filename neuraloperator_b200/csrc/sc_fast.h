@@ -15,11 +15,15 @@ bool fast_can_synthesize(const Plan* p, bool adjoint);
 // forward / backward chains: every operand access of the tensor-core contraction becomes contiguous along the image index
 // up to two contiguous global ranges the analysis launch pulls into L2 for the kernels that follow it (see AnaParams)
 struct L2Prefetch { const void* ptr[2] = {nullptr, nullptr}; unsigned long long bytes[2] = {0, 0}; };
+// storage: 0 = float images, SC_FLAG_GRID_F16 / SC_FLAG_GRID_BF16 = 16-bit images (the `float*` then addresses 16-bit data):
+// the forward analysis reads x that way when fast_analysis_reads_16bit(p), the adjoint synthesis writes dx that way
 bool fast_analyze(const Plan* p, const float* images, int64_t n_images, float2* modes_out, bool adjoint,
-                  cudaStream_t st, bool quad_major = false, const L2Prefetch* prefetch = nullptr);
+                  cudaStream_t st, bool quad_major = false, const L2Prefetch* prefetch = nullptr, int storage = 0);
+bool fast_analysis_reads_16bit(const Plan* p);
 // n_images counts the 2-D slices the fused kernel sees (images x dim-0 extent for 3-D problems)
 bool fast_synthesize(const Plan* p, const float2* modes_in, int64_t n_images, int n_channels, const float* bias,
-                     float* images_out, bool adjoint, int slices_per_image, cudaStream_t st, bool quad_major = false);
+                     float* images_out, bool adjoint, int slices_per_image, cudaStream_t st, bool quad_major = false,
+                     int storage = 0);
 int fast_tile_group(const Plan* p, bool synthesis, bool adjoint);   // slices per 128-row tile
 
 void fast_set_reserve(bool on);   // the next persistent transform launches of this thread leave plan->reserved_sms SMs free

@@ -5,6 +5,9 @@
 // (spectral_convolution.py:552-559) are all properties of the table, not of the kernel.  The tcgen05/TMA
 // path (sc_fast_*.cu) covers the large power-of-two shapes; this file is the path every other shape takes
 // and the cross-check for the fast one.  Compiled for sm_100a only.
+#include <algorithm>
+
+#include "sc_half.cuh"
 #include "sc_plan.h"
 
 namespace sc {
@@ -558,4 +561,79 @@ bool launch_bias_grad(const float2* gm, float* dbias, int batch, int out_channel
   return cuda_ok(cudaGetLastError(), "k_bias_grad launch");
 }
 
+// =====================================================================================================
+// 5. 16-bit image storage (SC_FLAG_GRID_F16 / SC_FLAG_GRID_BF16): x is widened to fp32 before the analysis, dx rounded to
+//    nearest even after the adjoint synthesis.  Widening is exact, so the transforms see the very values the fp32 path would.
+//    The element pair (sc_half.cuh) is shared with the tensor-core kernels and sc_hostcheck_convert.
+// =====================================================================================================
+constexpr int GC_THREADS = 256;
+constexpr int GC_VEC = 8;   // elements per vector step: 16 bytes of 16-bit data, 32 bytes of float
+
+// n_vec vector steps over 16-byte aligned buffers, then the scalar tail [8 n_vec, n)
+template <int G, bool TO16>
+__global__ void __launch_bounds__(GC_THREADS) k_grid_convert(const void* __restrict__ in, void* __restrict__ out, long long n,
+                                                             long long n_vec) {
+  const long long stride = (long long)gridDim.x * GC_THREADS;
+  for (long long v = (long long)blockIdx.x * GC_THREADS + threadIdx.x; v < n_vec; v += stride) {
+    if constexpr (TO16) {
+      const float4* src = reinterpret_cast<const float4*>(in) + 2 * v;
+      const float4 a = __ldg(src), b = __ldg(src + 1);
+      const float f[GC_VEC] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+      uint32_t w[4];
+#pragma unroll
+      for (int e = 0; e < 4; ++e) w[e] = (uint32_t)g16_store<G>(f[2 * e]) | ((uint32_t)g16_store<G>(f[2 * e + 1]) << 16);
+      reinterpret_cast<uint4*>(out)[v] = make_uint4(w[0], w[1], w[2], w[3]);
+    } else {
+      const uint4 q = __ldg(reinterpret_cast<const uint4*>(in) + v);
+      const uint32_t w[4] = {q.x, q.y, q.z, q.w};
+      float f[GC_VEC];
+#pragma unroll
+      for (int e = 0; e < 4; ++e) { f[2 * e] = g16_load<G>((uint16_t)(w[e] & 0xffffu)); f[2 * e + 1] = g16_load<G>((uint16_t)(w[e] >> 16)); }
+      float4* dst = reinterpret_cast<float4*>(out) + 2 * v;
+      dst[0] = make_float4(f[0], f[1], f[2], f[3]);
+      dst[1] = make_float4(f[4], f[5], f[6], f[7]);
+    }
+  }
+  for (long long i = GC_VEC * n_vec + (long long)blockIdx.x * GC_THREADS + threadIdx.x; i < n; i += stride) {
+    if constexpr (TO16) static_cast<uint16_t*>(out)[i] = g16_store<G>(static_cast<const float*>(in)[i]);
+    else static_cast<float*>(out)[i] = g16_load<G>(static_cast<const uint16_t*>(in)[i]);
+  }
+}
+
+bool launch_grid_convert(int grid16, const void* in, void* out, int64_t n, bool to_16, cudaStream_t st) {
+  if (n <= 0) return true;
+  if (grid16 != SC_FLAG_GRID_F16 && grid16 != SC_FLAG_GRID_BF16) { set_error("grid_convert: unknown 16-bit storage flag"); return false; }
+  const bool aligned = ((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out)) & 15u) == 0;
+  const long long n_vec = aligned ? (long long)(n / GC_VEC) : 0;
+  const long long work = n_vec > 0 ? n_vec : n;
+  const unsigned blocks = (unsigned)std::min<long long>((work + GC_THREADS - 1) / GC_THREADS, 148LL * 16);
+  if (grid16 == SC_FLAG_GRID_F16) {
+    if (to_16) k_grid_convert<SC_FLAG_GRID_F16, true><<<blocks, GC_THREADS, 0, st>>>(in, out, (long long)n, n_vec);
+    else k_grid_convert<SC_FLAG_GRID_F16, false><<<blocks, GC_THREADS, 0, st>>>(in, out, (long long)n, n_vec);
+  } else {
+    if (to_16) k_grid_convert<SC_FLAG_GRID_BF16, true><<<blocks, GC_THREADS, 0, st>>>(in, out, (long long)n, n_vec);
+    else k_grid_convert<SC_FLAG_GRID_BF16, false><<<blocks, GC_THREADS, 0, st>>>(in, out, (long long)n, n_vec);
+  }
+  count_launch();
+  return cuda_ok(cudaGetLastError(), "k_grid_convert launch");
+}
+
 }  // namespace sc
+
+extern "C" int sc_hostcheck_convert(int flag, int to_16, const void* in, void* out, int64_t n) {
+  using namespace sc;
+  if ((flag != SC_FLAG_GRID_F16 && flag != SC_FLAG_GRID_BF16) || n < 0 || (n > 0 && (in == nullptr || out == nullptr))) {
+    set_error("sc_hostcheck_convert: flag must be SC_FLAG_GRID_F16 or SC_FLAG_GRID_BF16, with n >= 0 elements");
+    return 1;
+  }
+  for (int64_t i = 0; i < n; ++i) {
+    if (to_16) {
+      const float f = static_cast<const float*>(in)[i];
+      static_cast<uint16_t*>(out)[i] = flag == SC_FLAG_GRID_F16 ? g16_store<SC_FLAG_GRID_F16>(f) : g16_store<SC_FLAG_GRID_BF16>(f);
+    } else {
+      const uint16_t b = static_cast<const uint16_t*>(in)[i];
+      static_cast<float*>(out)[i] = flag == SC_FLAG_GRID_F16 ? g16_load<SC_FLAG_GRID_F16>(b) : g16_load<SC_FLAG_GRID_BF16>(b);
+    }
+  }
+  return 0;
+}

@@ -52,6 +52,7 @@ struct Plan {
   bool fast_enabled = true;
   int reserved_sms = 0;                    // SMs the persistent transform kernels leave free (for a concurrent collective)
   bool host_only = false;                  // tables computed on the host only, nothing uploaded (sc_problem_table)
+  int grid16 = 0;                          // SC_FLAG_GRID_F16 / SC_FLAG_GRID_BF16: storage of x / dx, 0 = float
   std::vector<float> h_TA, h_TAT, h_TS, h_TST;   // host copies of the last-dim tables
   FastTables* fast = nullptr;              // tcgen05 path state (nullptr when the shape does not qualify)
   std::vector<void*> owned;                // every cudaMalloc made for this plan
@@ -88,6 +89,9 @@ bool launch_mode_gemm(ModeGemmOperand A, bool conjA, ModeGemmOperand B, bool con
                       int nR, int nC, int nK, int64_t nModes, cudaStream_t st);
 bool launch_bias_grad(const float2* gm, float* dbias, int batch, int out_channels, int64_t n_modes, int dc_slot,
                       float inv_scale, cudaStream_t st);
+// 16-bit image storage (grid16 = SC_FLAG_GRID_F16 / SC_FLAG_GRID_BF16): n elements 16-bit -> float (to_16 false) or float -> 16-bit
+// rounded to nearest even (to_16 true)
+bool launch_grid_convert(int grid16, const void* in, void* out, int64_t n, bool to_16, cudaStream_t st);
 
 // two-shot all-reduce (average) over NVLink peer memory, sc_collective.cu
 bool launch_allreduce_p2p(float* const* bufs, uint32_t* const* signals, int rank, int world, int64_t n_floats, float scale, int n_ctas,

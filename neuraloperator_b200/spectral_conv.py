@@ -58,6 +58,7 @@ class Plan:
         for k in self.kept:
             self.n_modes_total *= k
         self.max_n_modes = tuple(int(m) for m in max_n_modes)
+        self.grid_dtype = _GRID_DTYPES[int(flags) & (_lib.FLAG_GRID_F16 | _lib.FLAG_GRID_BF16)]   # x and dx; y / gy are float32
         self._bins = {}
         self._ws_bytes = {}
         self.plan_kept = None        # lazily: the same problem with weight extents == kept modes (factorized chains)
@@ -105,6 +106,10 @@ class Plan:
         except Exception:
             pass
 
+
+# storage of x / dx -> plan flag; the kernels compute in fp32 either way (a 16-bit value widens to float exactly)
+_GRID_FLAGS = {torch.float32: 0, torch.float16: _lib.FLAG_GRID_F16, torch.bfloat16: _lib.FLAG_GRID_BF16}
+_GRID_DTYPES = {flag: dtype for dtype, flag in _GRID_FLAGS.items()}
 
 _PLAN_CACHE: "OrderedDict[tuple, Plan]" = OrderedDict()
 _PLAN_LOCK = threading.RLock()      # re-entrant: building a ComplexPlan (under the lock) asks get_plan for its contraction plan
@@ -159,10 +164,11 @@ def _workspace(plan: Plan, n_images: int, device) -> torch.Tensor:
 # thin functional wrappers over the C ABI (also what the parity tests call)
 # --------------------------------------------------------------------------------------------------
 def analyze(plan: Plan, images: torch.Tensor, adjoint: bool = False) -> torch.Tensor:
-    """images (n0, n1, *grid) float32 -> kept modes (n0, n1, *kept) complex64 (adjoint: images on out_grid)."""
+    """images (n0, n1, *grid) in plan.grid_dtype -> kept modes (n0, n1, *kept) complex64 (adjoint: float32 images on out_grid)."""
     lib = _lib.load()
     spatial = plan.out_grid if adjoint else plan.grid
-    assert images.dtype == torch.float32 and images.is_contiguous() and tuple(images.shape[2:]) == spatial
+    dtype = torch.float32 if adjoint else plan.grid_dtype
+    assert images.dtype == dtype and images.is_contiguous() and tuple(images.shape[2:]) == spatial
     n_images = images.shape[0] * images.shape[1]
     modes = torch.empty((*images.shape[:2], *plan.kept), dtype=torch.complex64, device=images.device)
     ws = _workspace(plan, n_images, images.device)
@@ -173,11 +179,12 @@ def analyze(plan: Plan, images: torch.Tensor, adjoint: bool = False) -> torch.Te
 
 
 def synthesize(plan: Plan, modes: torch.Tensor, bias: Optional[torch.Tensor] = None, adjoint: bool = False) -> torch.Tensor:
+    """kept modes -> images: float32 on out_grid (+ bias), or with adjoint=True the gradient on grid in plan.grid_dtype."""
     lib = _lib.load()
     assert modes.dtype == torch.complex64 and modes.is_contiguous() and tuple(modes.shape[2:]) == plan.kept
     n_images = modes.shape[0] * modes.shape[1]
     spatial = plan.grid if adjoint else plan.out_grid
-    out = torch.empty((*modes.shape[:2], *spatial), dtype=torch.float32, device=modes.device)
+    out = torch.empty((*modes.shape[:2], *spatial), dtype=plan.grid_dtype if adjoint else torch.float32, device=modes.device)
     ws = _workspace(plan, n_images, modes.device)
     b = bias.reshape(-1).contiguous() if bias is not None else None
     with torch.cuda.device(modes.device):
@@ -230,6 +237,7 @@ class _SpectralConvDense(torch.autograd.Function):
         with torch.cuda.device(dev):
             _lib.check(lib.sc_forward_dense(plan.handle, _ptr(x), _ptr(weight), _ptr(b), _ptr(y), _ptr(xm), ctypes.byref(layout),
                                             B, Ci, Co, _ptr(ws), ws.numel(), _stream_ptr(dev)), "sc_forward_dense")
+        ctx.x_dtype = x.dtype            # dx is stored like x (16-bit image storage)
         ctx.saved_layout = int(layout.value)      # xm is opaque: the library says how it ordered the saved modes
         ctx.plan = plan
         ctx.reducer = reducer
@@ -251,7 +259,7 @@ class _SpectralConvDense(torch.autograd.Function):
         B, Ci = xm.shape[:2]
         Co = weight.shape[1]
         dev = gy.device
-        dx = torch.empty((B, Ci, *plan.grid), dtype=torch.float32, device=dev) if need_dx else None
+        dx = torch.empty((B, Ci, *plan.grid), dtype=ctx.x_dtype, device=dev) if need_dx else None
         if need_dw and need_db:
             # dweight and dbias share one allocation so that a data-parallel reducer moves them with ONE collective; a peer-memory
             # reducer hands out its symmetric buffer, so that the kernels write the gradients where the collective reads them
@@ -337,6 +345,7 @@ class _SpectralConvTucker(torch.autograd.Function):
             _lib.check(lib.sc_forward_tucker(plan.handle, plan_kept.handle, _ptr(x), _ptr(core), _ptr(u_in), _ptr(u_out), modes_ptrs, _ptr(b),
                                              _ptr(y), _ptr(saved), B, Ci, Co, ranks, _ptr(ws), ws.numel(), _stream_ptr(dev)),
                        "sc_forward_tucker")
+        ctx.x_dtype = x.dtype            # dx is stored like x (16-bit image storage)
         ctx.plan, ctx.plan_kept, ctx.d = plan, plan_kept, d
         ctx.bias_shape = bias.shape if bias is not None else None
         ctx.dims = (B, Ci, Co)
@@ -356,7 +365,7 @@ class _SpectralConvTucker(torch.autograd.Function):
         if gy.dtype != torch.float32:
             gy = gy.float()
         ranks, ws_bytes, _ = _SpectralConvTucker._args(plan, B, Ci, Co, core)
-        dx = torch.empty((B, Ci, *plan.grid), dtype=torch.float32, device=dev)
+        dx = torch.empty((B, Ci, *plan.grid), dtype=ctx.x_dtype, device=dev)
         d_core = torch.empty_like(core)
         d_u_in = torch.empty_like(u_in)
         d_u_out = torch.empty_like(u_out)
@@ -557,6 +566,7 @@ class _SpectralConvCPCall(torch.autograd.Function):
         with torch.cuda.device(dev):
             _lib.check(lib.sc_forward_cp(plan.handle, _ptr(x), _ptr(lam), _ptr(u_in), _ptr(u_out), _ptr_array(u_modes), _ptr(b), _ptr(y),
                                          _ptr(saved), B, Ci, Co, R, _ptr(ws), ws.numel(), _stream_ptr(dev)), "sc_forward_cp")
+        ctx.x_dtype = x.dtype            # dx is stored like x (16-bit image storage)
         ctx.plan = plan
         ctx.bias_shape = bias.shape if bias is not None else None
         ctx.dims = (B, Ci, Co, R)
@@ -575,7 +585,7 @@ class _SpectralConvCPCall(torch.autograd.Function):
         gy = gy.contiguous()
         if gy.dtype != torch.float32:
             gy = gy.float()
-        dx = torch.empty((B, Ci, *plan.grid), dtype=torch.float32, device=dev)
+        dx = torch.empty((B, Ci, *plan.grid), dtype=ctx.x_dtype, device=dev)
         d_lam, d_u_in, d_u_out = torch.empty_like(lam), torch.empty_like(u_in), torch.empty_like(u_out)
         d_modes = [torch.empty_like(u) for u in u_modes]
         db = torch.empty(Co, dtype=torch.float32, device=dev) if ctx.bias_shape is not None else None
@@ -611,6 +621,7 @@ class _SpectralConvTTCall(torch.autograd.Function):
         with torch.cuda.device(dev):
             _lib.check(lib.sc_forward_tt(plan.handle, plan_kept.handle, _ptr(x), _ptr(g0), _ptr(g1c), _ptr_array(cores), _ptr(b), _ptr(y),
                                          _ptr(saved), B, Ci, Co, ranks, _ptr(ws), ws.numel(), _stream_ptr(dev)), "sc_forward_tt")
+        ctx.x_dtype = x.dtype            # dx is stored like x (16-bit image storage)
         ctx.plan, ctx.plan_kept = plan, plan_kept
         ctx.bias_shape = bias.shape if bias is not None else None
         ctx.dims = (B, Ci, Co)
@@ -630,7 +641,7 @@ class _SpectralConvTTCall(torch.autograd.Function):
         if gy.dtype != torch.float32:
             gy = gy.float()
         ranks = _SpectralConvTTCall._ranks(g1c, cores)
-        dx = torch.empty((B, Ci, *plan.grid), dtype=torch.float32, device=dev)
+        dx = torch.empty((B, Ci, *plan.grid), dtype=ctx.x_dtype, device=dev)
         d_g0, d_g1 = torch.empty_like(g0), torch.empty_like(g1c)
         d_cores = [torch.empty_like(c) for c in cores]
         db = torch.empty(Co, dtype=torch.float32, device=dev) if ctx.bias_shape is not None else None
@@ -1154,8 +1165,18 @@ class SpectralConv(BaseSpectralConv):
             raise RuntimeError("neuraloperator_b200.SpectralConv has no CPU path: move the module and input to a B200")
         if self.complex_data:
             return self._forward_complex(x, output_shape)
-        if x.dtype != torch.float32:
-            raise TypeError(f"SpectralConv (full precision, real data) expects float32 input, got {x.dtype}")
+        if x.dtype not in _GRID_FLAGS:
+            raise TypeError(f"SpectralConv (real data) expects float32, float16 or bfloat16 input, got {x.dtype}")
+        if torch.is_autocast_enabled("cuda"):
+            # the result must not depend on autocast: a 16-bit x runs the 16-bit storage path, and nothing in between (a factorized
+            # weight's reconstruction, say) may be recast
+            with torch.autocast("cuda", enabled=False):
+                return self._forward_real(x, output_shape)
+        return self._forward_real(x, output_shape)
+
+    def _forward_real(self, x: torch.Tensor, output_shape):
+        """Real data in float32, float16 or bfloat16 (the lifting layer's output under torch.autocast): y is float32 whatever the
+        input dtype, as the reference's complex64 output spectrum makes it (:456-462); dx comes back in x's dtype."""
         # the kernels read the parameters through raw pointers: complex64 / float32 on x's device, nothing else
         for name, prm in self.named_parameters():
             want = torch.float32 if name == "bias" else torch.complex64
@@ -1166,15 +1187,18 @@ class SpectralConv(BaseSpectralConv):
                 raise RuntimeError(f"SpectralConv parameter {name} lives on {prm.device} but the input on {x.device}")
         grid = list(x.shape[2:])
         out_grid = self._output_grid(grid, output_shape)
-        plan = get_plan(x.device, grid, out_grid, self.n_modes, self.max_n_modes, self.fft_norm)
+        reduced = self.fno_block_precision != "full"
+        if reduced and x.dtype != torch.float32:
+            x = x.float()       # the reduced path rounds where the reference casts; autograd rounds dx back to x's dtype
+        plan = get_plan(x.device, grid, out_grid, self.n_modes, self.max_n_modes, self.fft_norm, flags=_GRID_FLAGS[x.dtype])
         if x.shape[0] == 0:
             # empty batch (torch.fft accepts it in the reference): nothing to launch; stay connected to the autograd graph
             z = x.sum() * 0
             for prm in self.parameters():
                 z = z + (prm.real.sum() if prm.is_complex() else prm.sum()) * 0
-            return x.new_zeros((0, self.out_channels, *out_grid)) + z
+            return x.new_zeros((0, self.out_channels, *out_grid), dtype=torch.float32) + z
         x = x.contiguous()
-        if self.fno_block_precision != "full":
+        if reduced:
             w = self.weight.to_tensor()
             return _SpectralConvDenseReduced.apply(x, w if w.is_contiguous() else w.contiguous(), self.bias, plan,
                                                    self.fno_block_precision == "half")
